@@ -4,7 +4,8 @@ oracle/ref_shim.py.  Run in the build container only (the GPU box has no /root/r
 
     python tests/golden/make_golden.py
 
-Outputs (small, committed): tests/golden/aggregation_golden.json, tests/golden/vq_golden.npz
+Outputs (small, committed): tests/golden/aggregation_golden.json, tests/golden/vq_golden.npz (read it through
+`load_vq_golden`)
 """
 from __future__ import annotations
 
@@ -117,8 +118,24 @@ def main() -> None:
         out[f"{tag}_dz"] = z.grad.numpy()
         out[f"{tag}_dE"] = vq.embedding.weight.grad.numpy()
         out[f"{tag}_usage"] = np.float64(vq.get_codebook_usage_percentage_from_indices(idx))
-    np.savez_compressed(os.path.join(HERE, "vq_golden.npz"), **out)
+    np.savez_compressed(os.path.join(HERE, "vq_golden.npz"), **{key: v for key, v in out.items() if not key.endswith("_dz")})
+    rebuilt = load_vq_golden()
+    for key, v in out.items():
+        assert np.array_equal(rebuilt[key], v) and rebuilt[key].dtype == v.dtype, f"{key} is not rebuilt bit for bit"
     print("wrote", os.listdir(HERE))
+
+
+def load_vq_golden() -> dict:
+    """tests/golden/vq_golden.npz as a dict.  Each tag's `dz` is left out of the file (it would take it over 1 MB) and
+    rebuilt here: the gradient `r` through the straight-through output plus 0.7 x the commitment loss' gradient
+    2 (z - E[idx]) / N, in float32.  main() checks that this equals the reference module's autograd bit for bit."""
+    gold = dict(np.load(os.path.join(HERE, "vq_golden.npz")))
+    for tag in ("init", "trained", "dup"):
+        z, E, r = gold[f"{tag}_z"], gold[f"{tag}_E"], gold[f"{tag}_r"]
+        B, D, H, W = z.shape
+        e = E[gold[f"{tag}_idx"]].reshape(B, H, W, D).transpose(0, 3, 1, 2)
+        gold[f"{tag}_dz"] = r + np.float32(0.7 * 2 / z.size) * (z - e)
+    return gold
 
 
 if __name__ == "__main__":

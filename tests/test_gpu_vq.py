@@ -8,14 +8,18 @@ own result depends on its BLAS accumulation order) -- those are counted and repo
 output bit-exact where the index agrees; losses / gradients within rtol 1e-5 / atol 1e-6 unless noted.
 """
 import os
+import sys
 
 import numpy as np
 import pytest
 import torch
 
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+from make_golden import load_vq_golden  # noqa: E402
+
 pytestmark = pytest.mark.gpu
 
-GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "vq_golden.npz"))
+GOLD = load_vq_golden()
 TAGS = ("init", "trained", "dup")
 
 

@@ -1,6 +1,7 @@
 """CPU tests: the VQ oracle restatement against golden outputs of the reference module
 (models/vq_vae.py:11-124 run behind the shim by tests/golden/make_golden.py)."""
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -8,7 +9,10 @@ import torch
 
 from oracle import vq as ov
 
-GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "vq_golden.npz"))
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+from make_golden import load_vq_golden  # noqa: E402
+
+GOLD = load_vq_golden()
 TAGS = ("init", "trained", "dup")
 
 
