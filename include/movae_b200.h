@@ -45,7 +45,7 @@ enum {
     MOVAE_DIAG_SIMILARITY = 0,   /* cos(J^T w, mean_rows J) from G alone; replaces main.py:94-122 */
     MOVAE_DIAG_COUNT = 1,        /* MGDA convergence_count (mgda.py:265) */
     MOVAE_DIAG_GAMMA = 2,        /* MGDA last gamma (mgda.py:266) */
-    MOVAE_DIAG_RANK = 3,         /* Aligned-MTL numerical rank (aligned_mtl.py:110) */
+    MOVAE_DIAG_RANK = 3,         /* Aligned-MTL numerical rank (aligned_mtl.py:110); IMTL-G: eigenvalues kept by the pseudo-inverse */
     MOVAE_DIAG_STATUS = 4,       /* 0 ok; 1 = QP residual above tolerance or non-finite weights (torchjd raises ValueError);
                                   * 2 = a peer's Gramian partial never arrived (the weights are NaN then) */
     MOVAE_DIAG_RESIDUAL = 5,     /* UPGrad: worst KKT violation over the k QPs */
@@ -116,9 +116,16 @@ int movae_recombine_f32(const float* d_J, int k, int64_t P, int64_t ldJ, const f
 
 /* ---- generic solve dispatch (same kernels as the four entry points above) -------------------- */
 enum { MOVAE_SOLVE_CONSTANT = 0, MOVAE_SOLVE_UPGRAD = 1, MOVAE_SOLVE_MGDA = 2, MOVAE_SOLVE_ALIGNED_MTL = 3, MOVAE_SOLVE_DUALPROJ = 4,
-       MOVAE_SOLVE_COMFORT = 5 };   /* utils/torchmoo/comfort.py:148-158: w = c0 * w_mgda + c1 * w_upgrad, {c0, c1} = d_aux = {1 - beta, beta}
+       MOVAE_SOLVE_COMFORT = 5,     /* utils/torchmoo/comfort.py:148-158: w = c0 * w_mgda + c1 * w_upgrad, {c0, c1} = d_aux = {1 - beta, beta}
                                      * as float32 in DEVICE memory (set_epoch rewrites it; a captured launch follows the schedule);
                                      * MGDA fields + norm_eps / reg_eps of the UPGrad half; d_w receives 2k values: the blend, then w_mgda */
+       MOVAE_SOLVE_PCGRAD = 6,      /* [torchjd] PCGradWeighting (selectable as `pcgrad`, main.py:1196-1220), float32: chain i starts at e_i
+                                     * and, for j in the order of row i of d_aux (float32 [k*k] DEVICE table, row i = a permutation of
+                                     * 0..k-1 drawn on the host, REQUIRED), subtracts its projection onto g_j when <g_j, J^T c> < 0;
+                                     * w = sum of the k chains.  A row that is not a permutation: STATUS 1 and NaN weights */
+       MOVAE_SOLVE_IMTLG = 7 };     /* [torchjd] IMTLGWeighting (`imtlg`): v = pinv(G) sqrt(diag G), eigenvalues |l| <= k eps32 max|l|
+                                     * dropped (pinv's default tolerance; d_diag[MOVAE_DIAG_RANK] = how many were kept), w = v / sum(v),
+                                     * w = 0 when |sum(v)| < 1e-12 */
 typedef struct movae_solve_spec {
     int32_t kind;                /* MOVAE_SOLVE_* */
     int32_t mode;                /* MGDA: norm_type; ALIGNED_MTL: scale_mode; UPGRAD: MOVAE_UPGRAD_NORM_* */
@@ -133,7 +140,8 @@ typedef struct movae_solve_spec {
 /* d_vec: pref vector (UPGRAD / DUALPROJ / ALIGNED_MTL, may be NULL) or losses (MGDA / COMFORT loss / loss+) */
 int movae_solve(const double* d_G, int k, const movae_solve_spec* spec, const float* d_vec, float* d_w,
                 double* d_diag, void* stream);
-/* same with the device-side auxiliary vector d_aux (COMFORT {1 - beta, beta}; UPGRAD with MOVAE_UPGRAD_NORM_DRAW {flag}) */
+/* same with the device-side auxiliary vector d_aux (COMFORT {1 - beta, beta}; UPGRAD with MOVAE_UPGRAD_NORM_DRAW {flag};
+ * PCGRAD the k x k permutation table) */
 int movae_solve_aux(const double* d_G, int k, const movae_solve_spec* spec, const float* d_vec, const float* d_aux, float* d_w,
                     double* d_diag, void* stream);
 

@@ -5,9 +5,9 @@ CUDA-only by design: importing works anywhere, but every op raises if the in-tre
 `mo-vae_b200/lib/libmovae_b200.so` is missing or the tensors are not on a CUDA device."""
 from . import ops, parallel  # noqa: F401
 from ._lib import LIB_PATH, lib  # noqa: F401
-from .aggregation import (COMFORT, MGDA, Aggregator, AlignedMTL, AlignedMTLWeighting, DualProj, GramianWeightedAggregator,  # noqa: F401
-                          Mean, MGDAWeighting, NUPGrad, PNUPGrad, StableMGDA, Sum, UPGrad, UPGradWeighting, Weighting,
-                          beta_schedule, make_aggregator)
+from .aggregation import (COMFORT, IMTLG, MGDA, Aggregator, AlignedMTL, AlignedMTLWeighting, DualProj,  # noqa: F401
+                          GramianWeightedAggregator, IMTLGWeighting, Mean, MGDAWeighting, NUPGrad, PCGrad, PCGradWeighting,
+                          PNUPGrad, StableMGDA, Sum, UPGrad, UPGradWeighting, Weighting, beta_schedule, make_aggregator)
 from .autojac import backward, mtl_backward  # noqa: F401
 from .extract import CodeExtractor  # noqa: F401
 from .host import HostAggregationPlan, aggregate_host  # noqa: F401

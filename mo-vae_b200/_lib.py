@@ -18,7 +18,7 @@ MGDA_NORM = {"none": 0, "l2": 1, "loss": 2, "loss+": 3}
 AMTL_SCALE = {"min": 0, "median": 1, "rmse": 2}
 UPGRAD_NORM = {"trace": 0, "min_l2": 1, "l2": 2, "draw": 3}
 
-SOLVE_CONSTANT, SOLVE_UPGRAD, SOLVE_MGDA, SOLVE_ALIGNED_MTL, SOLVE_DUALPROJ, SOLVE_COMFORT = range(6)
+SOLVE_CONSTANT, SOLVE_UPGRAD, SOLVE_MGDA, SOLVE_ALIGNED_MTL, SOLVE_DUALPROJ, SOLVE_COMFORT, SOLVE_PCGRAD, SOLVE_IMTLG = range(8)
 VQ_AUTO, VQ_EXACT, VQ_TENSOR = range(3)
 
 

@@ -10,6 +10,7 @@ Same names, constructor kwargs, call shape and error behaviour as the reference 
     MGDA(norm_type, epsilon, max_iters, stable, min_eigenvalue_eps), .set_losses(), .mgda_weighting
                                                                       (mgda.py:89-131)
     Sum(), Mean()                                                     (main.py:1198, :1223-1224)
+    PCGrad(), IMTLG()                                                 (torchjd; selectable at main.py:1196-1220)
 
 Every call is ONE fused launch (Gramian pass over J, small solve by the last CTA to arrive, recombination
 pass + write-back; csrc/aggregate.cu) on the current CUDA stream with no host synchronisation -- or, when a
@@ -54,8 +55,9 @@ class Weighting(nn.Module):
         """(movae_solve_spec, pref-or-losses tensor | None, device aux tensor | None) for the C entry points."""
         raise NotImplementedError
 
-    def prepare_step(self, device) -> None:
-        """Host-side per-step state that must reach the device BEFORE the launch (PNUPGrad's draw).  Default: nothing."""
+    def prepare_step(self, device, k: Optional[int] = None) -> None:
+        """Host-side per-step state that must reach the device BEFORE the launch of a k-row aggregation (PNUPGrad's and
+        PCGrad's draws).  Default: nothing."""
 
     def _select(self, w: Tensor, k: int) -> Tensor:
         """The weights this module reports out of the solve's output vector."""
@@ -75,7 +77,7 @@ class Weighting(nn.Module):
             return w
         ops.check_jacobian(matrix)
         matrix = matrix.detach()
-        self.prepare_step(matrix.device)
+        self.prepare_step(matrix.device, matrix.shape[0])
         if self.gramian_reducer is not None:
             G = ops.gram(matrix)
             self.gramian_reducer(G)
@@ -125,7 +127,7 @@ class Aggregator(nn.Module):
         """One launch; returns (weights used for the recombination, weights the weighting reports to its hooks)."""
         wt = self.weighting
         k = matrix.shape[0]
-        wt.prepare_step(matrix.device)
+        wt.prepare_step(matrix.device, k)
         spec, vec, aux = wt.solve_spec(k)
         w, diag, G, _ = ops.aggregate(matrix, spec, vec, aux, out=out, accumulate=accumulate, exchange=wt.p2p_exchange)
         return w[:k], (wt._select(w, k), diag, G)
@@ -142,7 +144,7 @@ class Aggregator(nn.Module):
         wt = self.weighting
         k = len(rows)
         dev = rows[0][0].device
-        wt.prepare_step(dev)
+        wt.prepare_step(dev, k)
         spec, vec, aux = wt.solve_spec(k)
         w, diag, G = ops.aggregate_segments(rows, numels, out_offsets, spec, vec, aux, out, accumulate, exchange=wt.p2p_exchange)
         wt.last_gramian, wt.last_diag = G, diag
@@ -274,20 +276,54 @@ class NUPGrad(Aggregator):
                 f"reg_eps={self._reg_eps}, solver={self._solver!r})")
 
 
-class _PNUPGradWeighting(UPGradWeighting):
+class _HostDraw:
+    """Mixin of the weightings whose solve consumes a per-aggregation draw from torch's default HOST generator, consumed
+    exactly as the reference consumes it.  The outcome is written into a fixed device buffer (`_aux`) that the solve reads
+    as d_aux, with stream-ordered writes, so a CUDA-graph replay follows the draws too: under capture the draw is deferred
+    to `GraphedStep`'s pre-replay callbacks (the captured launch only reads the buffer, which one eager run must have
+    created).  P-sharded / data-parallel: rank 0's draw is broadcast (`draw_group`, set by parallel.py; any installed
+    Gramian exchange implies the default group), all ranks must solve the same problem."""
+    _aux: Optional[Tensor] = None
+    draw_group = None                           # a process group (or True = the default one) whose rank 0's draw every rank uses
+
+    def _draw_into_device(self, device, k: Optional[int]) -> None:
+        raise NotImplementedError
+
+    def _device_buffer(self, n: int, device) -> Tensor:
+        if self._aux is None or self._aux.device != torch.device(device) or self._aux.numel() != n:
+            self._aux = torch.zeros(n, dtype=torch.float32, device=device)
+        return self._aux
+
+    def _broadcast_draw(self) -> None:
+        grp = self.draw_group
+        if grp is None and (self.p2p_exchange is not None or self.gramian_reducer is not None):
+            grp = True
+        if grp is not None:
+            import torch.distributed as dist
+            if dist.is_available() and dist.is_initialized() and dist.get_world_size(None if grp is True else grp) > 1:
+                dist.broadcast(self._aux, src=0, group=None if grp is True else grp)
+
+    def prepare_step(self, device, k: Optional[int] = None) -> None:
+        if torch.cuda.is_current_stream_capturing():
+            if self._aux is None:
+                raise RuntimeError(f"movae_b200: run {self._draw_owner} once eagerly before capturing it into a CUDA graph")
+            from .optim import register_pre_replay
+            register_pre_replay(lambda: self._draw_into_device(device, k))   # every replayed step draws on the host first
+            return
+        self._draw_into_device(device, k)
+
+
+class _PNUPGradWeighting(_HostDraw, UPGradWeighting):
     """utils/torchmoo/pnupgrad.py:127-134: with probability `prob` the cosine-normalised Gramian G / (|g_i||g_j|),
     otherwise NUPGrad's; the draw is `torch.rand(1).item() < prob` on the HOST RNG exactly like the reference, once per
-    aggregation.  Its outcome is written into a device flag the solve reads (MOVAE_UPGRAD_NORM_DRAW), so a CUDA-graph
-    replay follows the draws too: under capture the draw is deferred to `GraphedStep`'s pre-replay callbacks (the
-    captured launch only reads the flag).  P-sharded / data-parallel: rank 0's draw is broadcast, all ranks must solve
-    the same problem."""
+    aggregation.  Its outcome is a device flag the solve reads (MOVAE_UPGRAD_NORM_DRAW; _HostDraw carries it under CUDA
+    graphs and across ranks)."""
+    _draw_owner = "PNUPGrad"
 
     def __init__(self, pref_vector, prob: float, norm_eps: float, reg_eps: float, solver: str):
         super().__init__(pref_vector, norm_eps, reg_eps, solver)
         self.prob = prob
         self._mode = "min_l2"
-        self._flag: Optional[Tensor] = None      # float32 [1] on the device: 1.0 = the l2 branch was drawn
-        self.draw_group = None                   # set to a process group (or True) to broadcast rank 0's draw
 
     def _norm_mode(self) -> str:
         return "draw"
@@ -296,30 +332,16 @@ class _PNUPGradWeighting(UPGradWeighting):
         """One host draw; updates the device flag (a fill kernel carrying the value as an argument: race-free)."""
         self._mode = "l2" if torch.rand(1).item() < self.prob else "min_l2"
         if device is not None:
-            if self._flag is None or self._flag.device != torch.device(device):
-                self._flag = torch.zeros(1, dtype=torch.float32, device=device)
-            self._flag.fill_(1.0 if self._mode == "l2" else 0.0)
-            grp = self.draw_group
-            if grp is None and (self.p2p_exchange is not None or self.gramian_reducer is not None):
-                grp = True
-            if grp is not None:
-                import torch.distributed as dist
-                if dist.is_available() and dist.is_initialized() and dist.get_world_size(None if grp is True else grp) > 1:
-                    dist.broadcast(self._flag, src=0, group=None if grp is True else grp)
+            self._device_buffer(1, device).fill_(1.0 if self._mode == "l2" else 0.0)
+            self._broadcast_draw()
         return self._mode
 
-    def prepare_step(self, device) -> None:
-        if torch.cuda.is_current_stream_capturing():
-            if self._flag is None:
-                raise RuntimeError("movae_b200: run PNUPGrad once eagerly before capturing it into a CUDA graph")
-            from .optim import register_pre_replay
-            register_pre_replay(lambda: self.draw(device))    # the draw of every replayed step happens on the host, before it
-            return
+    def _draw_into_device(self, device, k: Optional[int]) -> None:
         self.draw(device)
 
     def solve_spec(self, k: int):
         spec, vec, _ = super().solve_spec(k)
-        return spec, vec, self._flag
+        return spec, vec, self._aux
 
 
 class PNUPGrad(Aggregator):
@@ -333,6 +355,73 @@ class PNUPGrad(Aggregator):
     def __repr__(self) -> str:
         return (f"{self.__class__.__name__}(pref_vector={self._pref_vector!r}, prob={self._prob}, norm_eps={self._norm_eps}, "
                 f"reg_eps={self._reg_eps}, solver={self._solver!r})")
+
+
+# ---- PCGrad / IMTL-G ------------------------------------------------------------------------------------
+class PCGradWeighting(_HostDraw, Weighting):
+    """torchjd `PCGradWeighting` [torchjd-recall] as a weighting of the Gramian: chain i starts at e_i and, in the order of
+    a fresh `torch.randperm(k)`, removes its conflict with every other row j (c_j -= <g_j, J^T c> / |g_j|^2 when that is
+    negative); w = the sum of the k chains, all float32 like torchjd's CPU loop.  The k permutations are drawn on the HOST
+    RNG exactly as torchjd draws them (k `torch.randperm(k)` calls per aggregation, row i first for chain i) and reach the
+    solve as a k x k device table."""
+    _draw_owner = "PCGrad"
+
+    def __init__(self):
+        super().__init__()
+        self.last_perms: Optional[Tensor] = None     # int64 [k, k] CPU: the permutations of the last draw
+
+    def draw(self, k: int, device=None) -> Tensor:
+        """One aggregation's draw: k `torch.randperm(k)` calls; with `device`, the table is copied into the device buffer
+        the solve reads (stream-ordered, from pinned memory the caching host allocator keeps until the copy has run)."""
+        self.last_perms = torch.stack([torch.randperm(k) for _ in range(k)])
+        if device is not None:
+            src = self.last_perms.to(torch.float32).reshape(-1).pin_memory()
+            self._device_buffer(k * k, device).copy_(src, non_blocking=True)
+            self._broadcast_draw()
+        return self.last_perms
+
+    def _draw_into_device(self, device, k: Optional[int]) -> None:
+        if k is None:
+            raise ValueError("movae_b200: PCGrad draws k permutations per aggregation; prepare_step needs k")
+        self.draw(k, device)
+
+    def solve_spec(self, k: int):
+        if self._aux is None or self._aux.numel() != k * k:
+            raise RuntimeError(f"movae_b200: no PCGrad permutation table for k={k} on the device (call prepare_step first)")
+        return L.SolveSpec(kind=L.SOLVE_PCGRAD), None, self._aux
+
+
+class PCGrad(Aggregator):
+    """Drop-in for torchjd.aggregation.PCGrad (selectable as `pcgrad`, main.py:1196-1220)."""
+
+    def __init__(self):
+        super().__init__(PCGradWeighting())
+
+    def __repr__(self) -> str:
+        return "PCGrad()"
+
+
+class IMTLGWeighting(Weighting):
+    """torchjd `IMTLGWeighting` [torchjd-recall]: v = pinv(G) sqrt(diag G), w = v / sum(v) (zeros when |sum(v)| < 1e-12),
+    the pseudo-inverse from a float64 eigen-decomposition with pinv's default tolerance (k eps32 max|eigenvalue|)."""
+
+    def solve_spec(self, k: int):
+        return L.SolveSpec(kind=L.SOLVE_IMTLG), None, None
+
+    @property
+    def rank(self) -> int:
+        """Eigenvalues of the Gramian the pseudo-inverse kept in the last solve."""
+        return int(self._diag(L.DIAG_RANK))
+
+
+class IMTLG(Aggregator):
+    """Drop-in for torchjd.aggregation.IMTLG (selectable as `imtlg`, main.py:1196-1220)."""
+
+    def __init__(self):
+        super().__init__(IMTLGWeighting())
+
+    def __repr__(self) -> str:
+        return "IMTLG()"
 
 
 # ---- Aligned-MTL ------------------------------------------------------------------------------------
@@ -608,9 +697,13 @@ def make_aggregator(name: Optional[str], *, agg_norm_eps: float = 1e-4, agg_reg_
         return PNUPGrad(norm_eps=agg_norm_eps, reg_eps=agg_reg_eps)
     if n == "comfort":
         return COMFORT(mgda_epsilon=mgda_epsilon, mgda_max_iters=mgda_max_iters, mgda_min_eigenvalue_eps=1e-10)
-    if n in ("pcgrad", "imtlg", "cagrad", "nashmtl"):
-        # selectable in the reference (main.py:1196-1220) but outside this path (SURVEY.md 2: random projections, an inner
-        # optimiser or cross-step state instead of Gramian -> weights -> J^T w): keep torchjd's aggregator for these
+    if n == "pcgrad":
+        return PCGrad()
+    if n == "imtlg":
+        return IMTLG()
+    if n in ("cagrad", "nashmtl"):
+        # selectable in the reference (main.py:1196-1220) but outside this path: CAGrad solves a cone program over the
+        # simplex (its result hangs on that solver's tolerances), NashMTL keeps optimiser state across steps
         raise ValueError(f"Aggregator {name} not supported by movae_b200 (not on the Gramian-weighting hot path); "
                          f"use torchjd.aggregation for it")
     raise ValueError(f"Aggregator {name} not supported")

@@ -8,6 +8,7 @@
 //               with >= 3 host syncs each (python `if c <= a`), normalisers :274-285, :319-367,
 //               eigen clamp :287-317
 //   * AlignedMTL: utils/torchmoo/aligned_mtl.py:97-133 -- cuSOLVER eigh on a k x k + host syncs
+//   * PCGrad / IMTL-G: torchjd PCGradWeighting (a float32 loop on the CPU) / IMTLGWeighting (torch.linalg.pinv)
 //   * the gradient-similarity hook main.py:94-122 (two more passes over J): here it is computed
 //     from G alone, 0 extra bytes.
 // Latency-bound by construction (k <= 8); excluded from GB/s, included in steps/s.
@@ -78,6 +79,12 @@ int fill_solve_params(int k, const movae_solve_spec* spec, SolveParams* out) {
             MOVAE_REQUIRE(p.scale_mode >= MOVAE_AMTL_MIN && p.scale_mode <= MOVAE_AMTL_RMSE, MOVAE_ERR_INVALID,
                           "aligned_mtl: bad scale_mode %d", p.scale_mode);
             break;
+        case MOVAE_SOLVE_PCGRAD:
+            p.kind = SOLVE_PCGRAD;
+            break;
+        case MOVAE_SOLVE_IMTLG:
+            p.kind = SOLVE_IMTLG;
+            break;
         default:
             set_error("solve: unknown kind %d", spec->kind);
             return MOVAE_ERR_INVALID;
@@ -92,6 +99,7 @@ int check_solve_vectors(const SolveParams& p, const float* d_vec, const float* d
     MOVAE_REQUIRE(!p.comfort || d_aux, MOVAE_ERR_INVALID, "comfort: the blend coefficients {1 - beta, beta} must be given (d_aux)");
     MOVAE_REQUIRE(!(p.kind == SOLVE_UPGRAD && p.upgrad_norm == MOVAE_UPGRAD_NORM_DRAW) || d_aux, MOVAE_ERR_INVALID,
                   "pnupgrad: the per-step draw flag must be given (d_aux)");
+    MOVAE_REQUIRE(p.kind != SOLVE_PCGRAD || d_aux, MOVAE_ERR_INVALID, "pcgrad: the k x k permutation table must be given (d_aux)");
     return MOVAE_OK;
 }
 
@@ -100,6 +108,8 @@ static int launch_solve(const SolveParams& p, const double* G, const float* vec,
     MOVAE_REQUIRE(G && w, MOVAE_ERR_INVALID, "solve: null pointer");
     const int rc = check_solve_vectors(p, vec, aux);
     if (rc != MOVAE_OK) return rc;
+    // the UPGrad QPs enumerate 2^k active sets, one per thread; every other solve runs on one or two warps (64 threads
+    // load the 8 x 8 Gramian)
     const int threads = (p.kind == SOLVE_UPGRAD || p.comfort) ? kSolveThreads : 64;
     solve_kernel<<<1, threads, 0, static_cast<cudaStream_t>(stream)>>>(p, G, vec, aux, w, diag);
     MOVAE_CUDA_TRY(cudaGetLastError());

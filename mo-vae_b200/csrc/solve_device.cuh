@@ -13,7 +13,7 @@ constexpr int MK = MOVAE_MAX_K;
 constexpr int kSolveThreads = 256;   // 2^MK active-set candidates for the UPGrad QPs
 constexpr float kEps32 = 1.1920928955078125e-07f;
 
-enum SolveKind { SOLVE_CONST = 0, SOLVE_UPGRAD = 1, SOLVE_MGDA = 2, SOLVE_AMTL = 3 };
+enum SolveKind { SOLVE_CONST = 0, SOLVE_UPGRAD = 1, SOLVE_MGDA = 2, SOLVE_AMTL = 3, SOLVE_PCGRAD = 4, SOLVE_IMTLG = 5 };
 
 struct SolveParams {
     int kind;
@@ -657,9 +657,91 @@ static __device__ __noinline__ void solve_amtl_part(const SolveParams& p, SolveS
     __syncthreads();
 }
 
+// PCGrad, torchjd PCGradWeighting op for op in float32: chain i starts at c = e_i and, for j in the order of row i of the
+// host-drawn permutation table `perm` (float32 [k*k]), j != i, computes ip = <G_j, c> and, when ip < 0, c_j -= ip / G_jj;
+// w = the k chains summed in order i = 0..k-1.  The chains are independent: lane i of warp 0 runs chain i, its c in a
+// row of shared memory (the indices come from the table).  A row that is not a permutation of 0..k-1 -> STATUS 1 and NaN
+// weights (check_status() raises instead of training on a corrupted draw).
+static __device__ __noinline__ void solve_pcgrad_part(const SolveParams& p, SolveSmem& S, const float* __restrict__ perm, int tid) {
+    const int k = p.k;
+    if (tid < 32) {
+        float (*C)[MK] = reinterpret_cast<float (*)[MK]>(&S.V[0][0]);     // V is unused by this solve
+        bool bad = false;
+        if (tid < k) {
+            const float* row = perm + tid * k;
+            unsigned seen = 0u;
+            for (int t = 0; t < k && !bad; ++t) {
+                const float v = row[t];
+                bad = !(v >= 0.f && v < (float)k) || (float)(int)v != v;
+                if (!bad) seen |= 1u << (int)v;
+            }
+            bad = bad || seen != (1u << k) - 1u;
+            for (int j = 0; j < k; ++j) C[tid][j] = (j == tid) ? 1.f : 0.f;
+            for (int t = 0; t < k && !bad; ++t) {
+                const int j = (int)row[t];
+                if (j == tid) continue;
+                float ip = 0.f;
+                for (int m = 0; m < k; ++m) ip = fmaf(S.Gf[j][m], C[tid][m], ip);
+                if (ip < 0.f) C[tid][j] = __fsub_rn(C[tid][j], __fdiv_rn(ip, S.Gf[j][j]));
+            }
+        }
+        bad = __any_sync(0xffffffffu, bad);
+        __syncwarp();
+        if (tid < k) {
+            float acc = 0.f;
+            for (int i = 0; i < k; ++i) acc = __fadd_rn(acc, C[i][tid]);
+            S.w[tid] = bad ? __int_as_float(0x7fc00000) : acc;
+        }
+        if (tid == 0 && bad) S.dg[MOVAE_DIAG_STATUS] = 1.0;
+    }
+    __syncthreads();
+}
+
+// IMTL-G, torchjd IMTLGWeighting: v = pinv(G) d with d = sqrt(diag G) (float32), w = v / sum(v), or 0 when |sum(v)| < 1e-12.
+// The pseudo-inverse of the symmetric G comes from the float64 Jacobi eigen-decomposition of the float32-rounded Gramian:
+// eigenvalues with |l| <= k eps32 max|l| are dropped (torch.linalg.pinv's default tolerance -- the singular values of a
+// symmetric matrix are the |l|), v = sum over the kept c of V_c (V_c . d) / l_c.  RANK = the number of kept eigenvalues.
+static __device__ __noinline__ void solve_imtlg_part(const SolveParams& p, SolveSmem& S, int tid) {
+    const int k = p.k;
+    if (tid < MK * MK) S.H[tid / MK][tid % MK] = (double)S.Gf[tid / MK][tid % MK];
+    __syncthreads();
+    if (tid < 32) {
+        jacobi_eigh_warp_rr(S.H, S.V, k, tid, S.rot_cs, S.rot_pq);
+        double amax = 0.0;
+        for (int c = 0; c < k; ++c) amax = fmax(amax, fabs(S.H[c][c]));
+        const double tol = amax * (double)k * (double)kEps32;
+        double* proj = &S.rot_cs[0][0];                            // k doubles of scratch (the rotations are done)
+        const bool kept = tid < k && fabs(S.H[tid][tid]) > tol;
+        if (tid < k) {                                             // lane c: (V_c . d) / l_c on eigenvector c
+            double pr = 0.0;
+            if (kept) {
+                for (int i = 0; i < k; ++i) pr += S.V[i][tid] * (double)__fsqrt_rn(S.Gf[i][i]);
+                pr /= S.H[tid][tid];
+            }
+            proj[tid] = pr;
+        }
+        const unsigned rank = __popc(__ballot_sync(0xffffffffu, kept));
+        __syncwarp();
+        if (tid < k) {                                             // lane i: component i of v
+            double o = 0.0;
+            for (int c = 0; c < k; ++c) o += S.V[tid][c] * proj[c];
+            S.lo[tid] = o;
+        }
+        __syncwarp();
+        if (tid < k) {
+            double s = 0.0;
+            for (int i = 0; i < k; ++i) s += S.lo[i];
+            S.w[tid] = (fabs(s) < 1e-12) ? 0.f : (float)(S.lo[tid] / s);
+        }
+        if (tid == 0) S.dg[MOVAE_DIAG_RANK] = (double)rank;
+    }
+    __syncthreads();
+}
+
 // The whole small solve.  Precondition: S.G holds the float64 Gramian (zero outside k x k) and every thread of the
 // CTA (blockDim.x >= 2^k for the UPGrad kinds, >= 64 otherwise) calls this.  `vec`: preference vector (UPGRAD /
-// DUALPROJ / AMTL, may be NULL) or losses (MGDA); `aux`: COMFORT {1 - beta, beta}, PNUPGrad {1.0 = l2 branch drawn}.
+// DUALPROJ / AMTL, may be NULL) or losses (MGDA); `aux`: COMFORT {1 - beta, beta}, PNUPGrad {1.0 = l2 branch drawn},
+// PCGrad the k x k permutation table.
 // `exchange_failed`: a peer's Gramian partial never arrived -> STATUS 2 and NaN weights (nothing downstream may
 // silently use a partial Gramian).  Postcondition: S.w[0..k) (COMFORT: S.w2 = the MGDA weights), S.dg.
 template <int KT>
@@ -690,6 +772,10 @@ __device__ __noinline__ void solve_block(const SolveParams& p, SolveSmem& S, con
         }
     } else if (p.kind == SOLVE_AMTL) {
         solve_amtl_part(p, S, vec, tid);
+    } else if (p.kind == SOLVE_PCGRAD) {
+        solve_pcgrad_part(p, S, aux, tid);
+    } else if (p.kind == SOLVE_IMTLG) {
+        solve_imtlg_part(p, S, tid);
     }
     __syncthreads();
 

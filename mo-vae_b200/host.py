@@ -70,7 +70,7 @@ class HostAggregationPlan:
                 gramian_reducer(bufs["G"])
             if hasattr(aggregator, "_ensure_coef"):
                 aggregator._ensure_coef(self.device)          # COMFORT: the blend coefficients live on the device
-            aggregator.weighting.prepare_step(self.device)
+            aggregator.weighting.prepare_step(self.device, k)
             spec, vec, aux = aggregator.weighting.solve_spec(k)
             vec = ops._dev_f32(vec, self.device, k, "pref_vector/losses")
             L.check(lib.movae_solve_aux(bufs["G"].data_ptr(), k, ctypes.byref(spec), L.ptr(vec), L.ptr(aux), bufs["w"].data_ptr(),

@@ -1,7 +1,8 @@
 """Aggregation microbench grid of BASELINE.json configs[4] on one GPU: k in {2,3,8} x P in {1e7,1e8,1e9}, every aggregator
 of north_star, each as ONE fused launch replayed from a CUDA graph of 10 (P = 1e7: rotating over 8 disjoint windows of a
-bigger Jacobian so that every launch is cold in L2) -> markdown table (profiles/r2_agg_sweep.md).
-    python tools/agg_sweep.py [--max-bytes 60e9]"""
+bigger Jacobian so that every launch is cold in L2) -> markdown table (profiles/r2_agg_sweep.md).  The graph is captured and
+replayed through GraphedStep, so aggregators with a per-step host draw (PCGrad, PNUPGrad) are timed with their draw.
+    python tools/agg_sweep.py [--max-bytes 60e9] [--names upgrad,pcgrad,imtlg]"""
 import argparse
 import json
 import os
@@ -16,6 +17,7 @@ from movae_b200 import ops  # noqa: E402
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--max-bytes", type=float, default=60e9)
+ap.add_argument("--names", default=None, help="comma-separated aggregator names for every (k, P); default: the north_star list")
 a = ap.parse_args()
 dev = torch.device("cuda")
 peak = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["hbm_gbs"] if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else 6650.0
@@ -40,6 +42,8 @@ for k in (2, 3, 8):
         out = torch.empty(Pa, dtype=torch.float32, device=dev)
         losses = torch.tensor([LOSSES[i % 5] for i in range(k)], device=dev)
         names = ("upgrad", "aligned_mtl", "aligned_mtl_median", "mgda_ln", "mgda_gn", "mgda_lgn", "jd_sum") if P < 1_000_000_000 else ("upgrad", "aligned_mtl")
+        if a.names:
+            names = tuple(a.names.split(","))
         for name in names:
             agg = movae_b200.make_aggregator(name)
             if isinstance(agg, movae_b200.MGDA):
@@ -47,24 +51,22 @@ for k in (2, 3, 8):
             Jw = [J[:, i * P:(i + 1) * P] for i in range(n_win)]
             ow = [out[i * P:(i + 1) * P] for i in range(n_win)]
             steps = 16 if n_win > 1 else 10
-            side = torch.cuda.Stream()
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                for i in range(2):
-                    agg.aggregate_into(Jw[i % n_win], ow[i % n_win])
-            torch.cuda.current_stream().wait_stream(side)
-            torch.cuda.synchronize()
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                ws = ops.current_workspace(J.device, k)
+            agg.aggregate_into(Jw[0], ow[0])                     # eager once: per-step device state (PCGrad's table) exists
+            captured = {}
+
+            def run_steps():
+                if torch.cuda.is_current_stream_capturing():
+                    captured["ws"] = ops.current_workspace(J.device, k)     # the capturing stream's workspace holds the stamps
                 for i in range(steps):
                     agg.aggregate_into(Jw[i % n_win], ow[i % n_win])
-            graph.replay()
+            graph = movae_b200.GraphedStep(run_steps, warmup=1)
+            ws = captured["ws"]
+            graph()
             best = 1e30
             for _ in range(3):
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
-                graph.replay()
+                graph()
                 e1.record()
                 torch.cuda.synchronize()
                 best = min(best, e0.elapsed_time(e1) / steps)
