@@ -267,6 +267,30 @@ int movae_vq_backward_f32(const float* d_grad_quantized, const float* d_g_commit
                           int64_t B, int D, int64_t HW, const float* d_E, int K, const int64_t* d_idx, float* d_dz, float* d_dE,
                           void* d_ws, size_t ws_bytes, void* stream);
 
+/* ---- exponential-moving-average codebook (VectorQuantizerEMA) --------------------------------- *
+ * Not the reference's rule: van den Oord et al. 2017 App. A.1 with the semantics of rosinality/vq-vae-2-pytorch `Quantize`.
+ * From the indices d_idx of the batch (searched with the pre-update codebook):
+ *     count_j = #{n : idx_n = j},  S_j = sum_{n : idx_n = j} z_n
+ *     cluster_size <- decay cluster_size + (1 - decay) count,   embed_avg <- decay embed_avg + (1 - decay) S
+ *     n = sum_j cluster_size_j,   E_j <- embed_avg_j / ((cluster_size_j + epsilon) / (n + K epsilon) n)
+ * E [K, D] is updated IN PLACE and d_E_prev [K, D] receives E as it was before the update.  d_cluster_size float32 [K],
+ * d_embed_avg float32 [K, D].  0 <= decay < 1, epsilon > 0 (else MOVAE_ERR_INVALID).  The workspace
+ * (movae_vq_ema_workspace_bytes, 16-byte aligned) is zero-filled ONCE before first use; the kernels leave it clean.
+ * movae_vq_ema_update_f32: the whole update.  K = 512, D = 64 (16-byte aligned E, embed_avg, E_prev): two launches,
+ * the statistics from K6b's partials, bit-reproducible; other shapes sum the rows with float32 atomics.
+ * The split pair, for a caller that reduces the statistics across data-parallel replicas in between:
+ * movae_vq_ema_stats_f32 writes d_stats float32 [K + K*D] = count, then S (row-major [K, D]); float32 counts are exact up
+ * to 2^24 rows per code (the fused update at K = 512, D = 64 counts in integers);
+ * movae_vq_ema_apply_f32 applies the EMA and the normalisation from such a d_stats. */
+size_t movae_vq_ema_workspace_bytes(int64_t n_rows, int K, int D);
+int movae_vq_ema_update_f32(const float* d_z, int64_t B, int D, int64_t HW, const int64_t* d_idx, int K, double decay, double epsilon,
+                            float* d_E, float* d_cluster_size, float* d_embed_avg, float* d_E_prev, void* d_ws, size_t ws_bytes,
+                            void* stream);
+int movae_vq_ema_stats_f32(const float* d_z, int64_t B, int D, int64_t HW, const int64_t* d_idx, int K, float* d_stats, void* d_ws,
+                           size_t ws_bytes, void* stream);
+int movae_vq_ema_apply_f32(const float* d_stats, int K, int D, double decay, double epsilon, float* d_E, float* d_cluster_size,
+                           float* d_embed_avg, float* d_E_prev, void* d_ws, size_t ws_bytes, void* stream);
+
 /* get_codebook_usage_percentage_from_indices (vq_vae.py:110-124): *d_count = |unique(idx)|. */
 int movae_vq_usage(const int64_t* d_idx, int64_t n, int K, int32_t* d_count, void* d_ws, size_t ws_bytes, void* stream);
 

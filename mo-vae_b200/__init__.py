@@ -12,6 +12,6 @@ from .autojac import backward, mtl_backward  # noqa: F401
 from .extract import CodeExtractor  # noqa: F401
 from .host import HostAggregationPlan, aggregate_host  # noqa: F401
 from .optim import (SGD, Adam, AdamW, FlatParameters, FusedOptimizer, GraphedStep, RMSprop, make_optimizer)  # noqa: F401
-from .quantizer import VectorQuantizer, code_indices, codebook_usage_count  # noqa: F401
+from .quantizer import VectorQuantizer, VectorQuantizerEMA, code_indices, codebook_usage_count  # noqa: F401
 
 __version__ = "0.1.0"

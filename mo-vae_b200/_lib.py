@@ -98,6 +98,12 @@ _SIGNATURES = {
     "movae_vq_backward_workspace_bytes": (c_size_t, [c_int64, c_int, c_int]),
     "movae_vq_backward_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int64, c_void_p, c_int,
                                       c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "movae_vq_ema_workspace_bytes": (c_size_t, [c_int64, c_int, c_int]),
+    "movae_vq_ema_update_f32": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_int, c_double, c_double, c_void_p, c_void_p,
+                                        c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "movae_vq_ema_stats_f32": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "movae_vq_ema_apply_f32": (c_int, [c_void_p, c_int, c_int, c_double, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                       c_size_t, c_void_p]),
     "movae_vq_usage": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "movae_vq_pack_codes": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "movae_vq_bitmap_count": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),

@@ -18,6 +18,13 @@ int launch_vq_pack_codes(const long long* idx, int64_t n, int K, void* out, int 
 int launch_vq_bitmap_count(const unsigned int* bitmap, int K, int* count, cudaStream_t st);
 int vq_backward_parts(int64_t n_rows, int K, int D);
 size_t vq_backward_part_bytes();
+size_t vq_ema_workspace_bytes(int64_t n_rows, int K, int D);
+int launch_vq_ema_stats(const float* z, int64_t N, int D, int64_t HW, const long long* idx, int K, float* stats, unsigned char* ws,
+                        cudaStream_t st);
+int launch_vq_ema_apply(const float* stats, int K, int D, double decay, double eps, float* E, float* cluster_size, float* embed_avg,
+                        float* E_prev, unsigned char* ws, cudaStream_t st);
+int launch_vq_ema_update(const float* z, int64_t N, int D, int64_t HW, const long long* idx, int K, double decay, double eps, float* E,
+                         float* cluster_size, float* embed_avg, float* E_prev, unsigned char* ws, cudaStream_t st);
 
 constexpr size_t kVqWsListOff = kWsListOff;
 constexpr int kVqMaxK = 65536;
@@ -27,6 +34,17 @@ static int check_shape(const char* what, int64_t B, int D, int64_t HW, int K) {
                   (long long)B, D, (long long)HW, K);
     MOVAE_REQUIRE(K <= kVqMaxK, MOVAE_ERR_UNSUPPORTED, "%s: num_embeddings %d > %d", what, K, kVqMaxK);
     MOVAE_REQUIRE(B * HW < ((int64_t)1 << 31), MOVAE_ERR_UNSUPPORTED, "%s: more than 2^31 code vectors", what);
+    return MOVAE_OK;
+}
+
+static int check_ema(const char* what, double decay, double eps, const float* E, const float* cs, const float* ea,
+                     const float* E_prev, const void* ws, size_t ws_bytes, size_t need) {
+    MOVAE_REQUIRE(decay >= 0.0 && decay < 1.0, MOVAE_ERR_INVALID, "%s: decay must be in [0, 1), got %g", what, decay);
+    MOVAE_REQUIRE(eps > 0.0, MOVAE_ERR_INVALID, "%s: epsilon must be > 0, got %g", what, eps);
+    MOVAE_REQUIRE(E && cs && ea && E_prev, MOVAE_ERR_INVALID, "%s: null pointer", what);
+    MOVAE_REQUIRE(E != E_prev && E != ea && ea != E_prev, MOVAE_ERR_INVALID, "%s: codebook, embed_avg and the pre-update copy must not alias", what);
+    MOVAE_REQUIRE(ws != nullptr && ws_bytes >= need, MOVAE_ERR_WORKSPACE, "%s: workspace too small (%zu < %zu)", what, ws_bytes, need);
+    MOVAE_REQUIRE(reinterpret_cast<uintptr_t>(ws) % 16 == 0, MOVAE_ERR_WORKSPACE, "%s: workspace must be 16-byte aligned", what);
     return MOVAE_OK;
 }
 
@@ -113,6 +131,53 @@ int movae_vq_backward_f32(const float* d_grad_quantized, const float* d_g_commit
     return launch_vq_backward(d_grad_quantized, d_g_commit, d_g_embed, d_z, N, D, HW, d_E, K,
                               reinterpret_cast<const long long*>(d_idx), d_dz, d_dE, need > 0 ? static_cast<float*>(d_ws) : nullptr,
                               static_cast<cudaStream_t>(stream));
+}
+
+size_t movae_vq_ema_workspace_bytes(int64_t n_rows, int K, int D) {
+    if (n_rows < 0 || K < 1 || K > movae::kVqMaxK || D < 1) return 0;
+    return movae::vq_ema_workspace_bytes(n_rows, K, D);
+}
+
+int movae_vq_ema_update_f32(const float* d_z, int64_t B, int D, int64_t HW, const int64_t* d_idx, int K, double decay, double epsilon,
+                            float* d_E, float* d_cluster_size, float* d_embed_avg, float* d_E_prev, void* d_ws, size_t ws_bytes,
+                            void* stream) {
+    using namespace movae;
+    int rc = check_shape("vq_ema_update", B, D, HW, K);
+    if (rc != MOVAE_OK) return rc;
+    const int64_t N = B * HW;
+    rc = check_ema("vq_ema_update", decay, epsilon, d_E, d_cluster_size, d_embed_avg, d_E_prev, d_ws, ws_bytes,
+                   movae_vq_ema_workspace_bytes(N, K, D));
+    if (rc != MOVAE_OK) return rc;
+    MOVAE_REQUIRE(N > 0, MOVAE_ERR_INVALID, "vq_ema_update: empty input (no code vector to average)");
+    MOVAE_REQUIRE(d_z && d_idx, MOVAE_ERR_INVALID, "vq_ema_update: null pointer");
+    return launch_vq_ema_update(d_z, N, D, HW, reinterpret_cast<const long long*>(d_idx), K, decay, epsilon, d_E, d_cluster_size,
+                                d_embed_avg, d_E_prev, static_cast<unsigned char*>(d_ws), static_cast<cudaStream_t>(stream));
+}
+
+int movae_vq_ema_stats_f32(const float* d_z, int64_t B, int D, int64_t HW, const int64_t* d_idx, int K, float* d_stats, void* d_ws,
+                           size_t ws_bytes, void* stream) {
+    using namespace movae;
+    const int rc = check_shape("vq_ema_stats", B, D, HW, K);
+    if (rc != MOVAE_OK) return rc;
+    const int64_t N = B * HW;
+    const size_t need = movae_vq_ema_workspace_bytes(N, K, D);
+    MOVAE_REQUIRE(d_stats && (N == 0 || (d_z && d_idx)), MOVAE_ERR_INVALID, "vq_ema_stats: null pointer");
+    MOVAE_REQUIRE(d_ws != nullptr && ws_bytes >= need, MOVAE_ERR_WORKSPACE, "vq_ema_stats: workspace too small (%zu < %zu)", ws_bytes, need);
+    MOVAE_REQUIRE(reinterpret_cast<uintptr_t>(d_ws) % 16 == 0, MOVAE_ERR_WORKSPACE, "vq_ema_stats: workspace must be 16-byte aligned");
+    return launch_vq_ema_stats(d_z, N, D, HW, reinterpret_cast<const long long*>(d_idx), K, d_stats, static_cast<unsigned char*>(d_ws),
+                               static_cast<cudaStream_t>(stream));
+}
+
+int movae_vq_ema_apply_f32(const float* d_stats, int K, int D, double decay, double epsilon, float* d_E, float* d_cluster_size,
+                           float* d_embed_avg, float* d_E_prev, void* d_ws, size_t ws_bytes, void* stream) {
+    using namespace movae;
+    MOVAE_REQUIRE(K >= 1 && K <= kVqMaxK && D >= 1, MOVAE_ERR_INVALID, "vq_ema_apply: bad shape K=%d D=%d", K, D);
+    const int rc = check_ema("vq_ema_apply", decay, epsilon, d_E, d_cluster_size, d_embed_avg, d_E_prev, d_ws, ws_bytes,
+                             movae_vq_ema_workspace_bytes(0, K, D));
+    if (rc != MOVAE_OK) return rc;
+    MOVAE_REQUIRE(d_stats != nullptr, MOVAE_ERR_INVALID, "vq_ema_apply: null pointer");
+    return launch_vq_ema_apply(d_stats, K, D, decay, epsilon, d_E, d_cluster_size, d_embed_avg, d_E_prev, static_cast<unsigned char*>(d_ws),
+                               static_cast<cudaStream_t>(stream));
 }
 
 int movae_vq_usage(const int64_t* d_idx, int64_t n, int K, int32_t* d_count, void* d_ws, size_t ws_bytes, void* stream) {

@@ -521,6 +521,7 @@ static int make_z_tensor_map(const float* z, int64_t B, int64_t HW, CUtensorMap*
 // thread (q, g) of a CTA sums the partials p = g, g + 4, g + 8, ... of output quad q (16-byte loads, 4 in flight), then the
 // four group sums are added in the order g = 0, 1, 2, 3 -- bit-reproducible, and 16 partial loads in flight per output
 // quad instead of 8 scalar ones per output element (the reduction of 148 partials was a 26 us latency chain).
+// ema_combine_partials (vq_ema.cu) repeats this combine for VectorQuantizerEMA: keep the two identical.
 constexpr int kRdGroups = 4, kRdQuads = 64, kRdThreads = kRdGroups * kRdQuads;
 __global__ void __launch_bounds__(kRdThreads)
 vq_dE_reduce_kernel(const float* __restrict__ partials, int n_parts, const float* __restrict__ g_embed,
@@ -583,6 +584,27 @@ int vq_backward_parts(int64_t n_rows, int K, int D) {
     return (int)(tiles < 160 ? tiles : 160);
 }
 
+// K6b's per-CTA partials (S [K, D] then the counts, kBwPartFloats each) for K = 512, D = 64: the tensor-map kernel when
+// 32-row boxes never straddle images and the copies are 16-byte aligned, else the cp.async one.  *n_parts = CTAs launched.
+// The caller has configured the kernels' dynamic shared memory on this device.
+int launch_k6b_partials(const float* z, int64_t N, int64_t HW, const long long* idx, float* partials, int* n_parts,
+                        cudaStream_t st) {
+    int grid = vq_backward_parts(N, kBwK, kBwD);
+    if (grid > sm_count()) grid = sm_count();
+    const bool tma_ok = (HW % 32 == 0) && reinterpret_cast<uintptr_t>(z) % 16 == 0 && reinterpret_cast<uintptr_t>(idx) % 16 == 0 &&
+                        HW * 4 * kBwD < ((int64_t)1 << 40);
+    if (tma_ok) {
+        CUtensorMap tmap;
+        const int rc = make_z_tensor_map(z, N / HW, HW, &tmap);
+        if (rc != MOVAE_OK) return rc;
+        vq_backward_dE_tma_kernel<<<grid, kTmThreads, kTmSmemBytes, st>>>(tmap, N, HW, idx, partials);
+    } else
+        vq_backward_dE_kernel<<<grid, kBwThreads, kBwSmemBytes, st>>>(z, N, HW, idx, partials);
+    MOVAE_CUDA_TRY(cudaGetLastError());
+    *n_parts = grid;
+    return MOVAE_OK;
+}
+
 int launch_vq_backward(const float* grad_out, const float* g_commit, const float* g_embed, const float* z, int64_t N, int D,
                        int64_t HW, const float* E, int K, const long long* idx, float* dz, float* dE, float* partials,
                        cudaStream_t st) {
@@ -611,19 +633,9 @@ int launch_vq_backward(const float* grad_out, const float* g_commit, const float
             MOVAE_CUDA_TRY(cudaGetLastError());
         }
         if (want_dE) {
-            int grid = vq_backward_parts(N, K, D);
-            if (grid > sms) grid = sms;
-            // tensor-map variant when 32-row boxes never straddle images and the copies are 16-byte aligned
-            const bool tma_ok = (HW % 32 == 0) && reinterpret_cast<uintptr_t>(z) % 16 == 0 && reinterpret_cast<uintptr_t>(idx) % 16 == 0 &&
-                                HW * 4 * kBwD < ((int64_t)1 << 40);
-            if (tma_ok) {
-                CUtensorMap tmap;
-                const int rc = make_z_tensor_map(z, N / HW, HW, &tmap);
-                if (rc != MOVAE_OK) return rc;
-                vq_backward_dE_tma_kernel<<<grid, kTmThreads, kTmSmemBytes, st>>>(tmap, N, HW, idx, partials);
-            } else
-                vq_backward_dE_kernel<<<grid, kBwThreads, kBwSmemBytes, st>>>(z, N, HW, idx, partials);
-            MOVAE_CUDA_TRY(cudaGetLastError());
+            int grid = 0;
+            const int rc = launch_k6b_partials(z, N, HW, idx, partials, &grid, st);
+            if (rc != MOVAE_OK) return rc;
             vq_dE_reduce_kernel<<<(K * D / 4 + kRdQuads - 1) / kRdQuads, kRdThreads, 0, st>>>(partials, grid, g_embed, E, N, dE);
             MOVAE_CUDA_TRY(cudaGetLastError());
         }
@@ -634,6 +646,19 @@ int launch_vq_backward(const float* grad_out, const float* g_commit, const float
     if (grid < 1) grid = 1;
     vq_backward_atomic_kernel<<<(unsigned)grid, 256, 0, st>>>(grad_out, g_commit, g_embed, z, N, D, HW, E, K, idx, dz, dE);
     MOVAE_CUDA_TRY(cudaGetLastError());
+    return MOVAE_OK;
+}
+
+// K6b's kernels need more than 48 KB of dynamic shared memory: configure them once per device (per host thread).
+int configure_k6b_partials() {
+    static thread_local int configured_dev = -1;
+    int dev = 0;
+    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
+    if (configured_dev != dev) {
+        MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_backward_dE_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwSmemBytes));
+        MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_backward_dE_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTmSmemBytes));
+        configured_dev = dev;
+    }
     return MOVAE_OK;
 }
 

@@ -50,6 +50,28 @@ def install_gramian_allreduce(aggregator: Aggregator, group: Optional[dist.Proce
     return aggregator
 
 
+def codebook_allreduce(group: Optional[dist.ProcessGroup] = None) -> Callable[[torch.Tensor], None]:
+    """In-place sum of a VectorQuantizerEMA's float32 [K + K*D] batch statistics (counts, then per-code sums) over the
+    process group: one collective, capturable into a CUDA graph on NCCL."""
+    def reduce_(stats: torch.Tensor) -> None:
+        if stats.dtype != torch.float32:
+            raise TypeError("the codebook statistics exchanged between ranks must be float32")
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+            dist.all_reduce(stats, op=dist.ReduceOp.SUM, group=group)
+    return reduce_
+
+
+def install_codebook_allreduce(vq, group: Optional[dist.ProcessGroup] = None):
+    """Makes the EMA update of `vq` (a VectorQuantizerEMA) use the statistics of the GLOBAL batch when every rank
+    quantizes its own slice of it: the counts and per-code sums are all-reduced between the statistics pass and the
+    update (as the all_reduce in rosinality's `Quantize`), so the replicas apply the same update and their codebooks stay
+    identical.  Returns `vq`."""
+    if not hasattr(vq, "stats_reducer"):
+        raise TypeError(f"install_codebook_allreduce needs a VectorQuantizerEMA, got {type(vq).__name__}")
+    vq.stats_reducer = codebook_allreduce(group)
+    return vq
+
+
 def check_replicated(t: torch.Tensor, group: Optional[dist.ProcessGroup] = None) -> bool:
     """True when `t` (e.g. the weights, or MGDA's losses) is bit-identical on every rank."""
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
