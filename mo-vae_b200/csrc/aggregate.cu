@@ -47,6 +47,31 @@ struct AggArgs {
     float* w_out;         // [k] (COMFORT: [2k], the MGDA weights second)
     double* diag_out;     // [MOVAE_DIAG_DOUBLES] or nullptr
     double* G_out;        // [k*k] summed Gramian, or nullptr
+    int64_t window_gram;  // L2 hand-off (below), in steps per CTA of the Gramian pass
+    int64_t window_rec;   //   and of the recombination pass
+};
+
+// ---- L2 hand-off of the tail of J from phase 1 to phase 3 ----------------------------------------------------------------
+// Phase 3 walks each CTA's deal in the reverse of phase 1's order, so the last steps of phase 1 are the first of phase 3.
+// The steps within `window` of the back of the deal (kL2WindowFraction of the L2 over the grid) are loaded evict_normal
+// by phase 1 and evict_first by phase 3, their last use in this launch.  Every other step is loaded evict_first by
+// phase 1, so that the bytes that are not reused in this launch do not push the window out of L2, and evict_normal by
+// phase 3: the front of J, which it reads last, is what the next launch's phase 1 reads first.  A weights-only launch
+// loads every step evict_normal, as K1 does.
+constexpr double kL2WindowFraction = 0.55;
+
+struct PolicyIO {
+    uint64_t pol;
+    __device__ __forceinline__ float4 load(const float4* p) const { return ld_stream_f4(p, pol); }
+    __device__ __forceinline__ float load(const float* p) const { return ld_stream_f1(p, pol); }
+};
+
+template <bool LAST_USE>
+struct WindowSteps {
+    int64_t window;
+    __device__ __forceinline__ PolicyIO operator()(int64_t d) const {
+        return {(d < window) == LAST_USE ? l2_policy_evict_first() : l2_policy_evict_normal()};
+    }
 };
 
 // Phase 2 of the fused launches, executed by the LAST CTA to arrive: fixed-order combine of the CTA partials, (multi-GPU) the
@@ -152,7 +177,7 @@ aggregate_kernel(AggArgs a, SolveParams sp, P2PArgs px) {
     double acc64[NACC];
 #pragma unroll
     for (int i = 0; i < NACC; ++i) acc64[i] = 0.0;
-    gram_stream_tiles<K, U1, VEC>(a.J, a.P, a.ldJ, acc64);
+    gram_stream_tiles<K, U1, VEC>(a.J, a.P, a.ldJ, acc64, WindowSteps<false>{a.window_gram});
     const bool last = gram_cta_partial_and_ticket<K>(acc64, partials, ticket, red, &is_last);
 
     // ---- phase 2 (last CTA to arrive): combine, exchange, solve, publish --------------------------------------------------
@@ -160,9 +185,9 @@ aggregate_kernel(AggArgs a, SolveParams sp, P2PArgs px) {
     if (a.out == nullptr) return;
 
     // ---- phase 3: recombine + write-back -----------------------------------------------------------------------------------
-    recombine_tiles<K, U2, VEC>(a.J, a.P, a.ldJ, a.w_out, a.out, a.accumulate, [&] {
-        if (!last) aggregate_wait_ready(ready, ready0);
-    });
+    recombine_tiles<K, U2, VEC>(
+        a.J, a.P, a.ldJ, a.w_out, a.out, a.accumulate, [&] { if (!last) aggregate_wait_ready(ready, ready0); },
+        WindowSteps<true>{a.window_rec});
     // end-of-launch timestamp by the last CTA to leave (diagnostics only)
     __syncthreads();
     if (tid == 0) {
@@ -176,12 +201,14 @@ aggregate_kernel(AggArgs a, SolveParams sp, P2PArgs px) {
 template <int K, int U1, int U2, bool VEC, int MINB>
 static int launch_aggregate(const AggArgs& a, const SolveParams& sp, const P2PArgs& px, cudaStream_t st) {
     auto kern = aggregate_kernel<K, U1, U2, VEC, MINB>;
-    static thread_local int occ_dev = -1, occ = 0;
+    constexpr int W = VEC ? 4 : 1;
+    static thread_local int occ_dev = -1, occ = 0, l2_bytes = 0;
     int dev = 0;
     MOVAE_CUDA_TRY(cudaGetDevice(&dev));
     if (occ_dev != dev) {
         MOVAE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kAggThreads, 0));
         if (occ < 1) occ = 1;
+        MOVAE_CUDA_TRY(cudaDeviceGetAttribute(&l2_bytes, cudaDevAttrL2CacheSize, dev));
         occ_dev = dev;
     }
     const int sms = sm_count();
@@ -194,6 +221,13 @@ static int launch_aggregate(const AggArgs& a, const SolveParams& sp, const P2PAr
     if (grid > n_tiles) grid = n_tiles;
     if (grid > kGramMaxBlocks) grid = kGramMaxBlocks;
     AggArgs a_ = a;
+    if (a.out != nullptr) {
+        const double window = kL2WindowFraction * (double)l2_bytes / (double)grid;    // bytes per CTA
+        a_.window_gram = (int64_t)(window / (double)((int64_t)K * kAggThreads * U1 * W * sizeof(float)));
+        a_.window_rec = (int64_t)(window / (double)((int64_t)K * kAggThreads * U2 * W * sizeof(float)));
+    } else {
+        a_.window_gram = a_.window_rec = INT64_MAX;
+    }
     SolveParams sp_ = sp;
     P2PArgs px_ = px;
     void* params[] = {&a_, &sp_, &px_};

@@ -41,6 +41,30 @@ __device__ __forceinline__ float ld_stream_f1(const float* p) {
     asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
     return v;
 }
+// The same loads with an L2 eviction priority.  The policy is a 64-bit descriptor from createpolicy; keep it warp-uniform
+// (it then travels in a uniform register: LDG.E.NA.128.CONSTANT desc[URx][...]).
+__device__ __forceinline__ uint64_t l2_policy_evict_first() {
+    uint64_t p;
+    asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
+    return p;
+}
+__device__ __forceinline__ uint64_t l2_policy_evict_normal() {
+    uint64_t p;
+    asm("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
+    return p;
+}
+__device__ __forceinline__ float4 ld_stream_f4(const float4* p, uint64_t pol) {
+    float4 v;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
+                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
+                 : "l"(p), "l"(pol));
+    return v;
+}
+__device__ __forceinline__ float ld_stream_f1(const float* p, uint64_t pol) {
+    float v;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(p), "l"(pol));
+    return v;
+}
 // streaming store (evict-first): the write-back is not re-read by this step
 __device__ __forceinline__ void st_stream_f4(float4* p, float4 v) {
     asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)

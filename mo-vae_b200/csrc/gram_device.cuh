@@ -53,10 +53,21 @@ __device__ __forceinline__ RRSchedule rr_schedule(int64_t n_items, int64_t tile_
     return s;
 }
 
+// How a pass loads one of a CTA's tiles: `steps(d)` gives the loader of the step d places from the back of the CTA's
+// deal (0: the remainder slice, or the last whole tile), in either pass.  K1 and K3 load every tile alike; the fused
+// kernel picks an L2 eviction priority per step (aggregate.cu).
+struct PlainTileIO {
+    __device__ __forceinline__ float4 load(const float4* p) const { return ld_stream_f4(p); }
+    __device__ __forceinline__ float load(const float* p) const { return ld_stream_f1(p); }
+};
+struct PlainSteps {
+    __device__ __forceinline__ PlainTileIO operator()(int64_t) const { return {}; }
+};
+
 // One tile of the Gramian pass: items [t0, t0 + tile) clipped to [t0, hi).
-template <int K, int U, bool VEC>
+template <int K, int U, bool VEC, class IO = PlainTileIO>
 __device__ __forceinline__ void gram_tile(const float* __restrict__ J, int64_t ldJ, int64_t t0, int64_t hi, bool full,
-                                          float (&acc)[GramAcc<K>::N]) {
+                                          float (&acc)[GramAcc<K>::N], IO io = {}) {
     const int64_t base = t0 + threadIdx.x;
     if constexpr (VEC) {
         float4 v[K][U];
@@ -65,14 +76,14 @@ __device__ __forceinline__ void gram_tile(const float* __restrict__ J, int64_t l
             for (int i = 0; i < K; ++i)
 #pragma unroll
                 for (int u = 0; u < U; ++u)
-                    v[i][u] = ld_stream_f4(reinterpret_cast<const float4*>(J + i * ldJ) + base + u * kGramThreads);
+                    v[i][u] = io.load(reinterpret_cast<const float4*>(J + i * ldJ) + base + u * kGramThreads);
         } else {
 #pragma unroll
             for (int i = 0; i < K; ++i)
 #pragma unroll
                 for (int u = 0; u < U; ++u) {
                     const int64_t idx = base + u * kGramThreads;
-                    v[i][u] = idx < hi ? ld_stream_f4(reinterpret_cast<const float4*>(J + i * ldJ) + idx)
+                    v[i][u] = idx < hi ? io.load(reinterpret_cast<const float4*>(J + i * ldJ) + idx)
                                        : make_float4(0.f, 0.f, 0.f, 0.f);
                 }
         }
@@ -99,7 +110,7 @@ __device__ __forceinline__ void gram_tile(const float* __restrict__ J, int64_t l
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const int64_t idx = base + u * kGramThreads;
-                v[i][u] = idx < hi ? ld_stream_f1(J + i * ldJ + idx) : 0.f;
+                v[i][u] = idx < hi ? io.load(J + i * ldJ + idx) : 0.f;
             }
 #pragma unroll
         for (int u = 0; u < U; ++u) {
@@ -113,9 +124,9 @@ __device__ __forceinline__ void gram_tile(const float* __restrict__ J, int64_t l
 
 // Streams this CTA's share of J front to back (rr_schedule over gridDim.x CTAs) and adds the products into acc64.
 // VEC: J base 16-byte aligned and ldJ % 4 == 0 -> float4 path; otherwise scalar path.
-template <int K, int U, bool VEC>
+template <int K, int U, bool VEC, class Steps = PlainSteps>
 __device__ __forceinline__ void gram_stream_tiles(const float* __restrict__ J, int64_t P, int64_t ldJ,
-                                                  double (&acc64)[GramAcc<K>::N]) {
+                                                  double (&acc64)[GramAcc<K>::N], Steps steps = {}) {
     constexpr int NACC = GramAcc<K>::N;
     constexpr int W = VEC ? 4 : 1;                       // columns per item
     constexpr int FLUSH = kGramChain / (W * U) > 0 ? kGramChain / (W * U) : 1;
@@ -123,6 +134,7 @@ __device__ __forceinline__ void gram_stream_tiles(const float* __restrict__ J, i
     const int64_t n_items = P / W;                       // float4 (or float) items per row
     constexpr int64_t tile_items = (int64_t)kGramThreads * U;
     const RRSchedule sch = rr_schedule(n_items, tile_items, blockIdx.x, gridDim.x);
+    const int64_t n_steps = sch.rounds + (sch.rem_hi > sch.rem_lo ? 1 : 0);
 
     int64_t r = 0;
     while (r < sch.rounds) {
@@ -132,7 +144,7 @@ __device__ __forceinline__ void gram_stream_tiles(const float* __restrict__ J, i
 #pragma unroll 1
         for (int f = 0; f < FLUSH && r < sch.rounds; ++f, ++r) {
             const int64_t t0 = (r * gridDim.x + blockIdx.x) * tile_items;
-            gram_tile<K, U, VEC>(J, ldJ, t0, t0 + tile_items, true, acc);
+            gram_tile<K, U, VEC>(J, ldJ, t0, t0 + tile_items, true, acc, steps(n_steps - 1 - r));
         }
 #pragma unroll
         for (int a = 0; a < NACC; ++a) acc64[a] += (double)acc[a];
@@ -141,7 +153,7 @@ __device__ __forceinline__ void gram_stream_tiles(const float* __restrict__ J, i
         float acc[NACC];
 #pragma unroll
         for (int a = 0; a < NACC; ++a) acc[a] = 0.f;
-        gram_tile<K, U, VEC>(J, ldJ, sch.rem_lo, sch.rem_hi, false, acc);
+        gram_tile<K, U, VEC>(J, ldJ, sch.rem_lo, sch.rem_hi, false, acc, steps(0));
 #pragma unroll
         for (int a = 0; a < NACC; ++a) acc64[a] += (double)acc[a];
     }

@@ -20,19 +20,19 @@ struct RecTile {
     T v[K][U];
 };
 
-template <int K, int U, bool VEC>
+template <int K, int U, bool VEC, class IO = PlainTileIO>
 __device__ __forceinline__ void rec_load_tile(RecTile<K, U, VEC>& r, const float* __restrict__ J, int64_t ldJ, int64_t base,
-                                              int64_t lo, int64_t hi, bool full) {
+                                              int64_t lo, int64_t hi, bool full, IO io = {}) {
 #pragma unroll
     for (int i = 0; i < K; ++i)
 #pragma unroll
         for (int u = 0; u < U; ++u) {
             const int64_t idx = base + u * kRecThreads;
             if constexpr (VEC)
-                r.v[i][u] = (full || (idx >= lo && idx < hi)) ? ld_stream_f4(reinterpret_cast<const float4*>(J + i * ldJ) + idx)
+                r.v[i][u] = (full || (idx >= lo && idx < hi)) ? io.load(reinterpret_cast<const float4*>(J + i * ldJ) + idx)
                                                     : make_float4(0.f, 0.f, 0.f, 0.f);
             else
-                r.v[i][u] = (full || (idx >= lo && idx < hi)) ? ld_stream_f1(J + i * ldJ + idx) : 0.f;
+                r.v[i][u] = (full || (idx >= lo && idx < hi)) ? io.load(J + i * ldJ + idx) : 0.f;
         }
 }
 
@@ -70,10 +70,10 @@ __device__ __forceinline__ void rec_store_tile(const RecTile<K, U, VEC>& r, cons
 // This CTA's share of the row (rr_schedule over gridDim.x CTAs, the same deal as the Gramian pass), BACK TO FRONT: first
 // its slice of the remainder region at the end of J, then its whole tiles in descending order.  Two register tiles: the
 // loads of the next tile are issued BEFORE the current one is combined and stored, so a thread never runs out of loads
-// in flight.
-template <int K, int U, bool VEC, class Ready>
+// in flight.  `steps` as in gram_stream_tiles: step i here is i places from the back of the deal.
+template <int K, int U, bool VEC, class Ready, class Steps = PlainSteps>
 __device__ __forceinline__ void recombine_tiles(const float* __restrict__ J, int64_t P, int64_t ldJ, const float* w_dev,
-                                                float* __restrict__ out, int accumulate, Ready ready) {
+                                                float* __restrict__ out, int accumulate, Ready ready, Steps steps = {}) {
     constexpr int W = VEC ? 4 : 1;
     const int tid = threadIdx.x;
     const int64_t n_items = P / W;
@@ -92,17 +92,17 @@ __device__ __forceinline__ void recombine_tiles(const float* __restrict__ J, int
     RecTile<K, U, VEC> ra, rb;
     int64_t i = 0;
     int64_t ta = 0, tb = 0;
-    if (n_steps > 0) { ta = t0_of(0); rec_load_tile<K, U, VEC>(ra, J, ldJ, ta + tid, ta, hi_of(0, ta), full_of(0)); }
+    if (n_steps > 0) { ta = t0_of(0); rec_load_tile<K, U, VEC>(ra, J, ldJ, ta + tid, ta, hi_of(0, ta), full_of(0), steps(0)); }
     ready();
     float w[K];
 #pragma unroll
     for (int q = 0; q < K; ++q) w[q] = __ldcg(w_dev + q);
     while (i < n_steps) {
         const bool has_b = i + 1 < n_steps;
-        if (has_b) { tb = t0_of(i + 1); rec_load_tile<K, U, VEC>(rb, J, ldJ, tb + tid, tb, hi_of(i + 1, tb), full_of(i + 1)); }
+        if (has_b) { tb = t0_of(i + 1); rec_load_tile<K, U, VEC>(rb, J, ldJ, tb + tid, tb, hi_of(i + 1, tb), full_of(i + 1), steps(i + 1)); }
         rec_store_tile<K, U, VEC>(ra, w, out, ta + tid, ta, hi_of(i, ta), full_of(i), accumulate);
         if (!has_b) break;
-        if (i + 2 < n_steps) { ta = t0_of(i + 2); rec_load_tile<K, U, VEC>(ra, J, ldJ, ta + tid, ta, hi_of(i + 2, ta), full_of(i + 2)); }
+        if (i + 2 < n_steps) { ta = t0_of(i + 2); rec_load_tile<K, U, VEC>(ra, J, ldJ, ta + tid, ta, hi_of(i + 2, ta), full_of(i + 2), steps(i + 2)); }
         rec_store_tile<K, U, VEC>(rb, w, out, tb + tid, tb, hi_of(i + 1, tb), full_of(i + 1), accumulate);
         i += 2;
     }
