@@ -174,7 +174,8 @@ typedef struct movae_jac_segments {
 int movae_aggregate_segments_f32(const movae_jac_segments* segs, const movae_solve_spec* spec, const float* d_vec,
                                  const float* d_aux, float* d_grad, int accumulate, float* d_w, double* d_diag, double* d_G,
                                  void* d_ws, size_t ws_bytes, const struct movae_p2p_ctx* ctx, void* stream);
-/* globaltimer stamps (ns) of the LAST movae_aggregate_f32 launch on this workspace: start, all partials in, weights
+/* globaltimer stamps (ns) of the LAST fused launch on this workspace (both movae_aggregate_f32 and
+ * movae_aggregate_segments_f32 write them): start, all partials in, weights
  * published, end, partials combined, exchange done -- how bench.py splits one launch into its two streaming passes and
  * the solve phase into its pieces.  Synchronises `stream`. */
 int movae_aggregate_timestamps(const void* d_ws, uint64_t h_stamps[6], void* stream);

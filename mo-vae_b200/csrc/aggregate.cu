@@ -22,9 +22,9 @@
 // argument (the exchange sequence number lives in the exchange buffer): the launch is CUDA-graph capturable.
 //
 // Roofline: HBM.  Algorithmic traffic 4*k*P (phase 1) + 4*k*P + 4*P (phase 3) bytes.
-// Workspace: movae_gram_workspace_bytes(k), zero-filled once; header: byte 0 ticket, 4 exit counter, 128 ready flag,
-// 192..255 timestamps of the last launch (globaltimer ns: start, all partials in, weights published, end, partials
-// combined, exchange done).
+// Workspace: movae_gram_workspace_bytes(k), zero-filled once; header layout: GramWorkspace (gram_device.cuh).  The
+// timestamps of the last launch are globaltimer ns: start, all partials in, weights published, end, partials combined,
+// exchange done.
 #include "recombine_device.cuh"
 #include "solve_device.cuh"
 
@@ -78,17 +78,16 @@ struct WindowSteps {
 // k x k exchange over peer memory, the small solve, publication of w through a release store on `ready`.
 template <int K>
 __device__ __forceinline__ void aggregate_solve_phase(const SolveParams& sp, const P2PArgs& px, const float* vec, const float* aux,
-                                                      float* w_out, double* diag_out, double* G_out, const double* partials,
-                                                      unsigned int* ticket, unsigned int* ready, unsigned int ready0,
-                                                      unsigned long long* stamps, unsigned long long t_start) {
+                                                      float* w_out, double* diag_out, double* G_out, const GramWorkspace& ws,
+                                                      unsigned int ready0, unsigned long long t_start) {
     __shared__ SolveSmem S;
     __shared__ double Gs[K * K];
     __shared__ unsigned long long seq_s;
     __shared__ int failed_s;
     const int tid = threadIdx.x;
     const unsigned long long t_in = global_timer_ns();
-    gram_combine_partials<K>(partials, Gs);
-    if (tid == 0) { *ticket = 0u; failed_s = 0; stamps[4] = global_timer_ns(); }   // self-reset: the workspace is reusable
+    gram_combine_partials<K>(ws.partials, Gs);
+    if (tid == 0) { *ws.ticket = 0u; failed_s = 0; ws.stamps[4] = global_timer_ns(); }   // self-reset: the workspace is reusable
     if (px.world > 0) {
         XchgBuffer* own = px.peers[px.rank];
         if (tid == 0) seq_s = own->step + 1;
@@ -114,7 +113,7 @@ __device__ __forceinline__ void aggregate_solve_phase(const SolveParams& sp, con
         }
         __syncthreads();
     }
-    if (tid == 0) stamps[5] = global_timer_ns();
+    if (tid == 0) ws.stamps[5] = global_timer_ns();
     if (tid < MK * MK) {
         const int i = tid / MK, j = tid % MK;
         S.G[i][j] = (i < K && j < K) ? Gs[i * K + j] : 0.0;
@@ -128,15 +127,24 @@ __device__ __forceinline__ void aggregate_solve_phase(const SolveParams& sp, con
     }
     __syncthreads();
     if (tid == 0) {
-        stamps[0] = t_start;
-        stamps[1] = t_in;
-        stamps[2] = global_timer_ns();
+        ws.stamps[0] = t_start;
+        ws.stamps[1] = t_in;
+        ws.stamps[2] = global_timer_ns();
         __threadfence();
-        st_release_gpu_u32(ready, ready0 + 1u);          // the other CTAs start their recombination pass now
+        st_release_gpu_u32(ws.ready, ready0 + 1u);         // the other CTAs start their recombination pass now
     }
     solve_diagnostics(sp, S, tid);                       // nobody waits for these
     __syncthreads();
     if (tid < MOVAE_DIAG_DOUBLES && diag_out) diag_out[tid] = S.dg[tid];
+}
+
+// Prologue of the fused launches, thread 0: the ready flag's value before this launch publishes its weights, and the start
+// stamp.
+__device__ __forceinline__ void aggregate_prologue(const GramWorkspace& ws, unsigned int& ready0, unsigned long long& t_start) {
+    if (threadIdx.x == 0) {
+        ready0 = ld_acquire_gpu_u32(ws.ready);
+        t_start = global_timer_ns();
+    }
 }
 
 // The other CTAs' wait for the weights (thread 0 polls, the CTA follows).
@@ -153,73 +161,61 @@ __device__ __forceinline__ void aggregate_wait_ready(const unsigned int* ready, 
     __syncthreads();
 }
 
+// Epilogue of the fused launches: the last CTA to leave stamps the end of the launch (diagnostics only).
+__device__ __forceinline__ void aggregate_epilogue(const GramWorkspace& ws) {
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        if (atomicAdd(ws.exit, 1u) == gridDim.x - 1) {
+            ws.stamps[3] = global_timer_ns();
+            *ws.exit = 0u;
+        }
+    }
+}
+
 template <int K, int U1, int U2, bool VEC, int MINB>
 __global__ void __launch_bounds__(kAggThreads, MINB)
 aggregate_kernel(AggArgs a, SolveParams sp, P2PArgs px) {
     constexpr int NACC = GramAcc<K>::N;
-    const int tid = threadIdx.x;
-    unsigned int* ticket = reinterpret_cast<unsigned int*>(a.ws);
-    unsigned int* done = reinterpret_cast<unsigned int*>(a.ws + 4);
-    unsigned int* ready = reinterpret_cast<unsigned int*>(a.ws + 128);
-    unsigned long long* stamps = reinterpret_cast<unsigned long long*>(a.ws + 192);
-    double* partials = reinterpret_cast<double*>(a.ws + kGramHeaderBytes);
-
+    const GramWorkspace ws(a.ws);
     __shared__ unsigned int ready0;
     __shared__ unsigned long long t_start;
     __shared__ double red[kGramThreads / 32][NACC];
     __shared__ int is_last;
-    if (tid == 0) {
-        ready0 = ld_acquire_gpu_u32(ready);      // the flag's value before this launch publishes its weights
-        t_start = global_timer_ns();
-    }
+    aggregate_prologue(ws, ready0, t_start);
 
     // ---- phase 1: Gramian partials ----------------------------------------------------------------------------------
     double acc64[NACC];
 #pragma unroll
     for (int i = 0; i < NACC; ++i) acc64[i] = 0.0;
     gram_stream_tiles<K, U1, VEC>(a.J, a.P, a.ldJ, acc64, WindowSteps<false>{a.window_gram});
-    const bool last = gram_cta_partial_and_ticket<K>(acc64, partials, ticket, red, &is_last);
+    const bool last = gram_cta_partial_and_ticket<K>(acc64, ws.partials, ws.ticket, red, &is_last);
 
     // ---- phase 2 (last CTA to arrive): combine, exchange, solve, publish --------------------------------------------------
-    if (last) aggregate_solve_phase<K>(sp, px, a.vec, a.aux, a.w_out, a.diag_out, a.G_out, partials, ticket, ready, ready0, stamps, t_start);
+    if (last) aggregate_solve_phase<K>(sp, px, a.vec, a.aux, a.w_out, a.diag_out, a.G_out, ws, ready0, t_start);
     if (a.out == nullptr) return;
 
     // ---- phase 3: recombine + write-back -----------------------------------------------------------------------------------
     recombine_tiles<K, U2, VEC>(
-        a.J, a.P, a.ldJ, a.w_out, a.out, a.accumulate, [&] { if (!last) aggregate_wait_ready(ready, ready0); },
+        a.J, a.P, a.ldJ, a.w_out, a.out, a.accumulate, [&] { if (!last) aggregate_wait_ready(ws.ready, ready0); },
         WindowSteps<true>{a.window_rec});
-    // end-of-launch timestamp by the last CTA to leave (diagnostics only)
-    __syncthreads();
-    if (tid == 0) {
-        if (atomicAdd(done, 1u) == gridDim.x - 1) {
-            stamps[3] = global_timer_ns();
-            *done = 0u;
-        }
-    }
+    aggregate_epilogue(ws);
 }
 
 template <int K, int U1, int U2, bool VEC, int MINB>
 static int launch_aggregate(const AggArgs& a, const SolveParams& sp, const P2PArgs& px, cudaStream_t st) {
-    auto kern = aggregate_kernel<K, U1, U2, VEC, MINB>;
+    constexpr auto kern = aggregate_kernel<K, U1, U2, VEC, MINB>;
     constexpr int W = VEC ? 4 : 1;
-    static thread_local int occ_dev = -1, occ = 0, l2_bytes = 0;
+    static thread_local int l2_dev = -1, l2_bytes = 0;
     int dev = 0;
     MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-    if (occ_dev != dev) {
-        MOVAE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kAggThreads, 0));
-        if (occ < 1) occ = 1;
+    if (l2_dev != dev) {
         MOVAE_CUDA_TRY(cudaDeviceGetAttribute(&l2_bytes, cudaDevAttrL2CacheSize, dev));
-        occ_dev = dev;
+        l2_dev = dev;
     }
-    const int sms = sm_count();
-    MOVAE_REQUIRE(sms > 0, MOVAE_ERR_CUDA, "CUDA device query failed (no GPU?)");
-    const int64_t n_items = a.P / (VEC ? 4 : 1);
     const int64_t tile_items = (int64_t)kAggThreads * (U1 > U2 ? U1 : U2);
-    int64_t n_tiles = (n_items + tile_items - 1) / tile_items;
-    if (n_tiles < 1) n_tiles = 1;
-    int64_t grid = (int64_t)sms * occ;       // every CTA must be resident: the CTAs wait for each other
-    if (grid > n_tiles) grid = n_tiles;
-    if (grid > kGramMaxBlocks) grid = kGramMaxBlocks;
+    unsigned int grid = 0;                   // every CTA must be resident: the CTAs wait for each other
+    const int rc = persistent_grid<kern>(kAggThreads, (a.P / W + tile_items - 1) / tile_items, kGramMaxBlocks, &grid);
+    if (rc != MOVAE_OK) return rc;
     AggArgs a_ = a;
     if (a.out != nullptr) {
         const double window = kL2WindowFraction * (double)l2_bytes / (double)grid;    // bytes per CTA
@@ -231,24 +227,8 @@ static int launch_aggregate(const AggArgs& a, const SolveParams& sp, const P2PAr
     SolveParams sp_ = sp;
     P2PArgs px_ = px;
     void* params[] = {&a_, &sp_, &px_};
-    MOVAE_CUDA_TRY(cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(kern), dim3((unsigned)grid), dim3(kAggThreads), params, 0, st));
+    MOVAE_CUDA_TRY(cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(kern), dim3(grid), dim3(kAggThreads), params, 0, st));
     return MOVAE_OK;
-}
-
-template <int K>
-static int dispatch_aggregate(const AggArgs& a, const SolveParams& sp, const P2PArgs& px, cudaStream_t st) {
-    const bool vec = (reinterpret_cast<uintptr_t>(a.J) % 16 == 0) && (a.out == nullptr || reinterpret_cast<uintptr_t>(a.out) % 16 == 0) &&
-                     (a.ldJ % 4 == 0 || K == 1);
-    // registers: float64 accumulators cost 2*K(K+1)/2; small k affords deeper unroll and 2 CTAs/SM
-    if (vec) {
-        if constexpr (K <= 2) return launch_aggregate<K, 8, 4, true, 2>(a, sp, px, st);
-        else if constexpr (K == 3) return launch_aggregate<K, 4, 4, true, 2>(a, sp, px, st);
-        else if constexpr (K == 4) return launch_aggregate<K, 4, 2, true, 2>(a, sp, px, st);     // two phase-3 register tiles of U2 = 4 spill at 128 regs
-        else return launch_aggregate<K, 2, 2, true, 1>(a, sp, px, st);
-    } else {
-        if constexpr (K <= 4) return launch_aggregate<K, 8, 8, false, 2>(a, sp, px, st);
-        else return launch_aggregate<K, 4, 4, false, 1>(a, sp, px, st);
-    }
 }
 
 // ---- segmented Jacobian: the rows are the gradient tensors autograd produced, wherever they live -----------------------
@@ -267,17 +247,19 @@ struct SegArgs {
     double* G_out;
 };
 
+// Row addressing of segment s (tile helpers, gram_device.cuh): its k row pointers, read from the kernel parameter.
+struct SegRows {
+    const float* const* rows;
+    __device__ __forceinline__ const float* row(int i) const { return rows[i]; }
+};
+
 template <int K, int U, int MINB>
 __global__ void __launch_bounds__(kAggThreads, MINB)
 aggregate_seg_kernel(const __grid_constant__ SegArgs a, SolveParams sp, P2PArgs px) {
     constexpr int NACC = GramAcc<K>::N;
     constexpr int kTile = kAggThreads * U;                 // float4 items per tile and row
     const int tid = threadIdx.x;
-    unsigned int* ticket = reinterpret_cast<unsigned int*>(a.ws);
-    unsigned int* done = reinterpret_cast<unsigned int*>(a.ws + 4);
-    unsigned int* ready = reinterpret_cast<unsigned int*>(a.ws + 128);
-    unsigned long long* stamps = reinterpret_cast<unsigned long long*>(a.ws + 192);
-    double* partials = reinterpret_cast<double*>(a.ws + kGramHeaderBytes);
+    const GramWorkspace ws(a.ws);
     const int n_seg = a.segs.n_segments;
 
     __shared__ unsigned int ready0;
@@ -285,9 +267,8 @@ aggregate_seg_kernel(const __grid_constant__ SegArgs a, SolveParams sp, P2PArgs 
     __shared__ double red[kGramThreads / 32][NACC];
     __shared__ int is_last;
     __shared__ int tile_start[MOVAE_MAX_SEGMENTS + 1];
+    aggregate_prologue(ws, ready0, t_start);
     if (tid == 0) {
-        ready0 = ld_acquire_gpu_u32(ready);
-        t_start = global_timer_ns();
         int acc = 0;
         for (int s = 0; s < n_seg; ++s) {
             tile_start[s] = acc;
@@ -299,160 +280,86 @@ aggregate_seg_kernel(const __grid_constant__ SegArgs a, SolveParams sp, P2PArgs 
     const int n_tiles = tile_start[n_seg];
     auto segment_of = [&](int v) { int s = 0; while (v >= tile_start[s + 1]) ++s; return s; };
 
-    // ---- phase 1 ----
+    // ---- phase 1: every tile is a float32 chain of its own, promoted into acc64 ----
     double acc64[NACC];
 #pragma unroll
     for (int i = 0; i < NACC; ++i) acc64[i] = 0.0;
     for (int v = blockIdx.x; v < n_tiles; v += gridDim.x) {
         const int s = segment_of(v);
-        const int64_t n_items = a.segs.n[s] >> 2;
-        const int64_t base = (int64_t)(v - tile_start[s]) * kTile + tid;
-        float4 x[K][U];
-#pragma unroll
-        for (int i = 0; i < K; ++i) {
-            const float4* row = reinterpret_cast<const float4*>(a.segs.rows[s][i]);
-#pragma unroll
-            for (int u = 0; u < U; ++u) {
-                const int64_t idx = base + u * kAggThreads;
-                x[i][u] = idx < n_items ? ld_stream_f4(row + idx) : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-        }
         float acc[NACC];
 #pragma unroll
         for (int q = 0; q < NACC; ++q) acc[q] = 0.f;
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            float c[K];
-#pragma unroll
-            for (int i = 0; i < K; ++i) c[i] = x[i][u].x;
-            gram_fma<K>(acc, c);
-#pragma unroll
-            for (int i = 0; i < K; ++i) c[i] = x[i][u].y;
-            gram_fma<K>(acc, c);
-#pragma unroll
-            for (int i = 0; i < K; ++i) c[i] = x[i][u].z;
-            gram_fma<K>(acc, c);
-#pragma unroll
-            for (int i = 0; i < K; ++i) c[i] = x[i][u].w;
-            gram_fma<K>(acc, c);
-        }
+        gram_tile<K, U, true>(SegRows{a.segs.rows[s]}, (int64_t)(v - tile_start[s]) * kTile, a.segs.n[s] >> 2, false, acc);
 #pragma unroll
         for (int q = 0; q < NACC; ++q) acc64[q] += (double)acc[q];
     }
     // ragged tails: columns 4 * (n / 4) .. n - 1 of every segment, one thread each in CTA 0
     if (blockIdx.x == 0 && tid < 4 * n_seg) {
-        const int s = tid >> 2, e = tid & 3;
-        const int64_t c0 = a.segs.n[s] & ~(int64_t)3;
-        if (c0 + e < a.segs.n[s]) {
-            float c[K];
-            float acc[NACC];
-#pragma unroll
-            for (int q = 0; q < NACC; ++q) acc[q] = 0.f;
-#pragma unroll
-            for (int i = 0; i < K; ++i) c[i] = a.segs.rows[s][i][c0 + e];
-            gram_fma<K>(acc, c);
-#pragma unroll
-            for (int q = 0; q < NACC; ++q) acc64[q] += (double)acc[q];
-        }
+        const int s = tid >> 2;
+        const int64_t c = (a.segs.n[s] & ~(int64_t)3) + (tid & 3);
+        if (c < a.segs.n[s]) gram_column<K>(SegRows{a.segs.rows[s]}, c, acc64);
     }
-    const bool last = gram_cta_partial_and_ticket<K>(acc64, partials, ticket, red, &is_last);
+    const bool last = gram_cta_partial_and_ticket<K>(acc64, ws.partials, ws.ticket, red, &is_last);
 
     // ---- phase 2 ----
-    if (last) aggregate_solve_phase<K>(sp, px, a.vec, a.aux, a.w_out, a.diag_out, a.G_out, partials, ticket, ready, ready0, stamps, t_start);
+    if (last) aggregate_solve_phase<K>(sp, px, a.vec, a.aux, a.w_out, a.diag_out, a.G_out, ws, ready0, t_start);
     if (a.out == nullptr) return;
 
-    // ---- phase 3: the virtual tiles back to front ----
+    // ---- phase 3: the virtual tiles back to front, one register tile ----
+    auto wait = [&] { if (!last) aggregate_wait_ready(ws.ready, ready0); };
     float w[K];
     bool have_w = false;
     for (int v = n_tiles - 1 - (int)blockIdx.x; v >= 0; v -= gridDim.x) {
         const int s = segment_of(v);
-        const int64_t n_items = a.segs.n[s] >> 2;
-        const int64_t base = (int64_t)(v - tile_start[s]) * kTile + tid;
-        float4 x[K][U];
-#pragma unroll
-        for (int i = 0; i < K; ++i) {
-            const float4* row = reinterpret_cast<const float4*>(a.segs.rows[s][i]);
-#pragma unroll
-            for (int u = 0; u < U; ++u) {
-                const int64_t idx = base + u * kAggThreads;
-                x[i][u] = idx < n_items ? ld_stream_f4(row + idx) : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-        }
+        const int64_t t0 = (int64_t)(v - tile_start[s]) * kTile, n_items = a.segs.n[s] >> 2;
+        RecTile<K, U, true> r;
+        rec_load_tile<K, U, true>(r, SegRows{a.segs.rows[s]}, t0 + tid, t0, n_items, false);
         if (!have_w) {
-            if (!last) aggregate_wait_ready(ready, ready0);
-#pragma unroll
-            for (int i = 0; i < K; ++i) w[i] = __ldcg(a.w_out + i);
+            rec_read_weights<K>(a.w_out, wait, w);
             have_w = true;
         }
-        float4* dst = reinterpret_cast<float4*>(a.out + a.segs.out_off[s]);
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const int64_t idx = base + u * kAggThreads;
-            if (idx >= n_items) continue;
-            float4 o;
-            o.x = w[0] * x[0][u].x; o.y = w[0] * x[0][u].y; o.z = w[0] * x[0][u].z; o.w = w[0] * x[0][u].w;
-#pragma unroll
-            for (int i = 1; i < K; ++i) {
-                o.x = fmaf(w[i], x[i][u].x, o.x); o.y = fmaf(w[i], x[i][u].y, o.y);
-                o.z = fmaf(w[i], x[i][u].z, o.z); o.w = fmaf(w[i], x[i][u].w, o.w);
-            }
-            if (a.accumulate) {
-                const float4 old = dst[idx];
-                o.x += old.x; o.y += old.y; o.z += old.z; o.w += old.w;
-            }
-            st_stream_f4(dst + idx, o);
-        }
+        rec_store_tile<K, U, true>(r, w, a.out + a.segs.out_off[s], t0 + tid, t0, n_items, false, a.accumulate);
     }
-    if (!have_w) {                                           // a CTA without tiles still has to join the protocol
-        if (!last) aggregate_wait_ready(ready, ready0);
-#pragma unroll
-        for (int i = 0; i < K; ++i) w[i] = __ldcg(a.w_out + i);
-    }
+    if (!have_w) rec_read_weights<K>(a.w_out, wait, w);      // a CTA without tiles still has to join the protocol
     if (blockIdx.x == 0 && tid < 4 * n_seg) {
-        const int s = tid >> 2, e = tid & 3;
-        const int64_t c = (a.segs.n[s] & ~(int64_t)3) + e;
-        if (c < a.segs.n[s]) {
-            float o = w[0] * a.segs.rows[s][0][c];
-#pragma unroll
-            for (int i = 1; i < K; ++i) o = fmaf(w[i], a.segs.rows[s][i][c], o);
-            float* dst = a.out + a.segs.out_off[s] + c;
-            *dst = a.accumulate ? *dst + o : o;
-        }
+        const int s = tid >> 2;
+        const int64_t c = (a.segs.n[s] & ~(int64_t)3) + (tid & 3);
+        if (c < a.segs.n[s]) rec_column<K>(SegRows{a.segs.rows[s]}, w, a.out + a.segs.out_off[s], c, a.accumulate);
     }
-    __syncthreads();
-    if (tid == 0) {
-        if (atomicAdd(done, 1u) == gridDim.x - 1) {
-            stamps[3] = global_timer_ns();
-            *done = 0u;
-        }
-    }
+    aggregate_epilogue(ws);
 }
 
 template <int K, int U, int MINB>
 static int launch_aggregate_seg(const SegArgs& a, const SolveParams& sp, const P2PArgs& px, cudaStream_t st) {
-    auto kern = aggregate_seg_kernel<K, U, MINB>;
-    static thread_local int occ_dev = -1, occ = 0;
-    int dev = 0;
-    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-    if (occ_dev != dev) {
-        MOVAE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kAggThreads, 0));
-        if (occ < 1) occ = 1;
-        occ_dev = dev;
-    }
-    const int sms = sm_count();
-    MOVAE_REQUIRE(sms > 0, MOVAE_ERR_CUDA, "CUDA device query failed (no GPU?)");
+    constexpr auto kern = aggregate_seg_kernel<K, U, MINB>;
     int64_t n_tiles = 0;
     for (int s = 0; s < a.segs.n_segments; ++s) n_tiles += ((a.segs.n[s] >> 2) + kAggThreads * U - 1) / (kAggThreads * U);
-    if (n_tiles < 1) n_tiles = 1;
-    int64_t grid = (int64_t)sms * occ;
-    if (grid > n_tiles) grid = n_tiles;
-    if (grid > kGramMaxBlocks) grid = kGramMaxBlocks;
+    unsigned int grid = 0;
+    const int rc = persistent_grid<kern>(kAggThreads, n_tiles, kGramMaxBlocks, &grid);
+    if (rc != MOVAE_OK) return rc;
     SegArgs a_ = a;
     SolveParams sp_ = sp;
     P2PArgs px_ = px;
     void* params[] = {&a_, &sp_, &px_};
-    MOVAE_CUDA_TRY(cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(kern), dim3((unsigned)grid), dim3(kAggThreads), params, 0, st));
+    MOVAE_CUDA_TRY(cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(kern), dim3(grid), dim3(kAggThreads), params, 0, st));
     return MOVAE_OK;
+}
+
+// Validation shared by the fused entry points, in this order: the solve spec and its vectors, the entry's own arguments
+// (check_args), the workspace (size, and 8-byte alignment for the float64 partials), the peer-to-peer context.
+template <class CheckArgs>
+static int check_fused_launch(const char* who, int k, const movae_solve_spec* spec, const float* d_vec, const float* d_aux,
+                              CheckArgs check_args, const void* d_ws, size_t ws_bytes, const movae_p2p_ctx* ctx, SolveParams* sp,
+                              P2PArgs* px) {
+    int rc = fill_solve_params(k, spec, sp);
+    if (rc == MOVAE_OK) rc = check_solve_vectors(*sp, d_vec, d_aux);
+    if (rc == MOVAE_OK) rc = check_args();
+    if (rc != MOVAE_OK) return rc;
+    MOVAE_REQUIRE(d_ws != nullptr && ws_bytes >= movae_gram_workspace_bytes(k), MOVAE_ERR_WORKSPACE,
+                  "%s: workspace too small (%zu < %zu)", who, ws_bytes, movae_gram_workspace_bytes(k));
+    MOVAE_REQUIRE(reinterpret_cast<uintptr_t>(d_ws) % 8 == 0, MOVAE_ERR_WORKSPACE, "%s: workspace must be 8-byte aligned", who);
+    *px = p2p_disabled();
+    return ctx != nullptr ? make_p2p_args(ctx, px) : MOVAE_OK;
 }
 
 }  // namespace movae
@@ -464,20 +371,13 @@ int movae_aggregate_f32(const float* d_J, int k, int64_t P, int64_t ldJ, const m
                         size_t ws_bytes, const movae_p2p_ctx* ctx, void* stream) {
     using namespace movae;
     SolveParams sp;
-    int rc = fill_solve_params(k, spec, &sp);
+    P2PArgs px;
+    const int rc = check_fused_launch("aggregate", k, spec, d_vec, d_aux, [&] {
+        MOVAE_REQUIRE(P >= 0 && ldJ >= P, MOVAE_ERR_INVALID, "aggregate: need 0 <= P <= ldJ (P=%lld ldJ=%lld)", (long long)P, (long long)ldJ);
+        MOVAE_REQUIRE(d_w != nullptr && (d_J != nullptr || P == 0), MOVAE_ERR_INVALID, "aggregate: null pointer");
+        return MOVAE_OK;
+    }, d_ws, ws_bytes, ctx, &sp, &px);
     if (rc != MOVAE_OK) return rc;
-    rc = check_solve_vectors(sp, d_vec, d_aux);
-    if (rc != MOVAE_OK) return rc;
-    MOVAE_REQUIRE(P >= 0 && ldJ >= P, MOVAE_ERR_INVALID, "aggregate: need 0 <= P <= ldJ (P=%lld ldJ=%lld)", (long long)P, (long long)ldJ);
-    MOVAE_REQUIRE(d_w != nullptr && (d_J != nullptr || P == 0), MOVAE_ERR_INVALID, "aggregate: null pointer");
-    MOVAE_REQUIRE(d_ws != nullptr && ws_bytes >= movae_gram_workspace_bytes(k), MOVAE_ERR_WORKSPACE,
-                  "aggregate: workspace too small (%zu < %zu)", ws_bytes, movae_gram_workspace_bytes(k));
-    MOVAE_REQUIRE(reinterpret_cast<uintptr_t>(d_ws) % 8 == 0, MOVAE_ERR_WORKSPACE, "aggregate: workspace must be 8-byte aligned");
-    P2PArgs px = p2p_disabled();
-    if (ctx != nullptr) {
-        rc = make_p2p_args(ctx, &px);
-        if (rc != MOVAE_OK) return rc;
-    }
     AggArgs a;
     a.J = d_J;
     a.P = P;
@@ -491,16 +391,21 @@ int movae_aggregate_f32(const float* d_J, int k, int64_t P, int64_t ldJ, const m
     a.diag_out = d_diag;
     a.G_out = d_G;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    switch (k) {
-        case 1: return dispatch_aggregate<1>(a, sp, px, st);
-        case 2: return dispatch_aggregate<2>(a, sp, px, st);
-        case 3: return dispatch_aggregate<3>(a, sp, px, st);
-        case 4: return dispatch_aggregate<4>(a, sp, px, st);
-        case 5: return dispatch_aggregate<5>(a, sp, px, st);
-        case 6: return dispatch_aggregate<6>(a, sp, px, st);
-        case 7: return dispatch_aggregate<7>(a, sp, px, st);
-        default: return dispatch_aggregate<8>(a, sp, px, st);
-    }
+    const bool vec = (reinterpret_cast<uintptr_t>(d_J) % 16 == 0) && (d_grad == nullptr || reinterpret_cast<uintptr_t>(d_grad) % 16 == 0) &&
+                     (ldJ % 4 == 0 || k == 1);
+    // registers: float64 accumulators cost 2*K(K+1)/2; small k affords deeper unroll and 2 CTAs/SM
+    return dispatch_k(k, [&](auto kc) {
+        constexpr int K = decltype(kc)::value;
+        if (vec) {
+            if constexpr (K <= 2) return launch_aggregate<K, 8, 4, true, 2>(a, sp, px, st);
+            else if constexpr (K == 3) return launch_aggregate<K, 4, 4, true, 2>(a, sp, px, st);
+            else if constexpr (K == 4) return launch_aggregate<K, 4, 2, true, 2>(a, sp, px, st);     // two phase-3 register tiles of U2 = 4 spill at 128 regs
+            else return launch_aggregate<K, 2, 2, true, 1>(a, sp, px, st);
+        } else {
+            if constexpr (K <= 4) return launch_aggregate<K, 8, 8, false, 2>(a, sp, px, st);
+            else return launch_aggregate<K, 4, 4, false, 1>(a, sp, px, st);
+        }
+    });
 }
 
 int movae_aggregate_segments_f32(const movae_jac_segments* segs, const movae_solve_spec* spec, const float* d_vec,
@@ -510,29 +415,23 @@ int movae_aggregate_segments_f32(const movae_jac_segments* segs, const movae_sol
     MOVAE_REQUIRE(segs != nullptr, MOVAE_ERR_INVALID, "aggregate_segments: null segment table");
     const int k = segs->k;
     SolveParams sp;
-    int rc = fill_solve_params(k, spec, &sp);
+    P2PArgs px;
+    const int rc = check_fused_launch("aggregate_segments", k, spec, d_vec, d_aux, [&] {
+        MOVAE_REQUIRE(segs->n_segments >= 1 && segs->n_segments <= MOVAE_MAX_SEGMENTS, MOVAE_ERR_UNSUPPORTED,
+                      "aggregate_segments: %d segments outside 1..%d", segs->n_segments, MOVAE_MAX_SEGMENTS);
+        MOVAE_REQUIRE(d_w != nullptr, MOVAE_ERR_INVALID, "aggregate_segments: null pointer");
+        MOVAE_REQUIRE(d_grad == nullptr || reinterpret_cast<uintptr_t>(d_grad) % 16 == 0, MOVAE_ERR_INVALID,
+                      "aggregate_segments: the gradient buffer must be 16-byte aligned");
+        for (int s = 0; s < segs->n_segments; ++s) {
+            MOVAE_REQUIRE(segs->n[s] >= 0 && segs->out_off[s] >= 0 && segs->out_off[s] % 4 == 0, MOVAE_ERR_INVALID,
+                          "aggregate_segments: segment %d needs n >= 0 and an output offset that is a multiple of 4", s);
+            for (int i = 0; i < k; ++i)
+                MOVAE_REQUIRE(segs->rows[s][i] != nullptr && reinterpret_cast<uintptr_t>(segs->rows[s][i]) % 16 == 0, MOVAE_ERR_INVALID,
+                              "aggregate_segments: row %d of segment %d must be a 16-byte aligned device pointer", i, s);
+        }
+        return MOVAE_OK;
+    }, d_ws, ws_bytes, ctx, &sp, &px);
     if (rc != MOVAE_OK) return rc;
-    rc = check_solve_vectors(sp, d_vec, d_aux);
-    if (rc != MOVAE_OK) return rc;
-    MOVAE_REQUIRE(segs->n_segments >= 1 && segs->n_segments <= MOVAE_MAX_SEGMENTS, MOVAE_ERR_UNSUPPORTED,
-                  "aggregate_segments: %d segments outside 1..%d", segs->n_segments, MOVAE_MAX_SEGMENTS);
-    MOVAE_REQUIRE(d_w != nullptr, MOVAE_ERR_INVALID, "aggregate_segments: null pointer");
-    MOVAE_REQUIRE(d_grad == nullptr || reinterpret_cast<uintptr_t>(d_grad) % 16 == 0, MOVAE_ERR_INVALID,
-                  "aggregate_segments: the gradient buffer must be 16-byte aligned");
-    for (int s = 0; s < segs->n_segments; ++s) {
-        MOVAE_REQUIRE(segs->n[s] >= 0 && segs->out_off[s] >= 0 && segs->out_off[s] % 4 == 0, MOVAE_ERR_INVALID,
-                      "aggregate_segments: segment %d needs n >= 0 and an output offset that is a multiple of 4", s);
-        for (int i = 0; i < k; ++i)
-            MOVAE_REQUIRE(segs->rows[s][i] != nullptr && reinterpret_cast<uintptr_t>(segs->rows[s][i]) % 16 == 0, MOVAE_ERR_INVALID,
-                          "aggregate_segments: row %d of segment %d must be a 16-byte aligned device pointer", i, s);
-    }
-    MOVAE_REQUIRE(d_ws != nullptr && ws_bytes >= movae_gram_workspace_bytes(k), MOVAE_ERR_WORKSPACE,
-                  "aggregate_segments: workspace too small (%zu < %zu)", ws_bytes, movae_gram_workspace_bytes(k));
-    P2PArgs px = p2p_disabled();
-    if (ctx != nullptr) {
-        rc = make_p2p_args(ctx, &px);
-        if (rc != MOVAE_OK) return rc;
-    }
     SegArgs a;
     a.segs = *segs;
     a.ws = static_cast<unsigned char*>(d_ws);
@@ -544,23 +443,20 @@ int movae_aggregate_segments_f32(const movae_jac_segments* segs, const movae_sol
     a.diag_out = d_diag;
     a.G_out = d_G;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    switch (k) {
-        case 1: return launch_aggregate_seg<1, 4, 2>(a, sp, px, st);
-        case 2: return launch_aggregate_seg<2, 4, 2>(a, sp, px, st);
-        case 3: return launch_aggregate_seg<3, 4, 2>(a, sp, px, st);
-        case 4: return launch_aggregate_seg<4, 2, 2>(a, sp, px, st);
-        case 5: return launch_aggregate_seg<5, 2, 1>(a, sp, px, st);
-        case 6: return launch_aggregate_seg<6, 2, 1>(a, sp, px, st);
-        case 7: return launch_aggregate_seg<7, 2, 1>(a, sp, px, st);
-        default: return launch_aggregate_seg<8, 2, 1>(a, sp, px, st);
-    }
+    return dispatch_k(k, [&](auto kc) {
+        constexpr int K = decltype(kc)::value;
+        if constexpr (K <= 3) return launch_aggregate_seg<K, 4, 2>(a, sp, px, st);
+        else if constexpr (K == 4) return launch_aggregate_seg<K, 2, 2>(a, sp, px, st);
+        else return launch_aggregate_seg<K, 2, 1>(a, sp, px, st);
+    });
 }
 
 int movae_aggregate_timestamps(const void* d_ws, uint64_t h_stamps[6], void* stream) {
     using namespace movae;
     MOVAE_REQUIRE(d_ws != nullptr && h_stamps != nullptr, MOVAE_ERR_INVALID, "aggregate_timestamps: null pointer");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    MOVAE_CUDA_TRY(cudaMemcpyAsync(h_stamps, static_cast<const unsigned char*>(d_ws) + 192, 6 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    MOVAE_CUDA_TRY(cudaMemcpyAsync(h_stamps, static_cast<const unsigned char*>(d_ws) + GramWorkspace::kStamps, 6 * sizeof(uint64_t),
+                                   cudaMemcpyDeviceToHost, st));
     MOVAE_CUDA_TRY(cudaStreamSynchronize(st));
     return MOVAE_OK;
 }

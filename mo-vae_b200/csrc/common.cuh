@@ -5,6 +5,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "../../include/movae_b200.h"
 
 namespace movae {
@@ -27,6 +29,35 @@ int sm_count();                                    // cached multiProcessorCount
             return (code);                      \
         }                                       \
     } while (0)
+
+// Grid of a persistent launch of `kern` with `threads` threads per CTA: as many CTAs as the device holds at once (SMs x
+// occupancy), at most one per tile and at most `cap`.  The occupancy is cached per kernel instantiation, host thread and
+// device: a cache keyed on the kernel's type alone would mix up the instantiations that share one.
+template <auto kern>
+int persistent_grid(int threads, int64_t n_tiles, int64_t cap, unsigned int* grid) {
+    static thread_local int occ_dev = -1, occ = 0;
+    int dev = 0;
+    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
+    if (occ_dev != dev) {
+        MOVAE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, 0));
+        if (occ < 1) occ = 1;
+        occ_dev = dev;
+    }
+    const int sms = sm_count();
+    MOVAE_REQUIRE(sms > 0, MOVAE_ERR_CUDA, "CUDA device query failed (no GPU?)");
+    int64_t g = (int64_t)sms * occ;
+    if (g > n_tiles) g = n_tiles;
+    if (g > cap) g = cap;
+    *grid = g > 1 ? (unsigned int)g : 1u;
+    return MOVAE_OK;
+}
+
+// Returns f(std::integral_constant<int, K>{}) for K = k; k is 1 .. MOVAE_MAX_K (larger k take MOVAE_MAX_K).
+template <int K = 1, class F>
+int dispatch_k(int k, F&& f) {
+    if constexpr (K == MOVAE_MAX_K) return f(std::integral_constant<int, K>{});
+    else return k == K ? f(std::integral_constant<int, K>{}) : dispatch_k<K + 1>(k, f);
+}
 
 // 128-bit streaming load: read-only path, do not allocate in L1 (each byte is used once per pass)
 __device__ __forceinline__ float4 ld_stream_f4(const float4* p) {

@@ -42,43 +42,15 @@ gram_kernel(const float* __restrict__ J, int64_t P, int64_t ldJ, double* __restr
 
 template <int K, int U, bool VEC, int MINB>
 static int launch_gram(const float* J, int64_t P, int64_t ldJ, double* G, int accumulate, void* ws, cudaStream_t st) {
-    auto kern = gram_kernel<K, U, VEC, MINB>;
-    static thread_local int occ_dev = -1, occ = 0;      // cached per (host thread, device)
-    int dev = 0;
-    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-    if (occ_dev != dev) {
-        MOVAE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kGramThreads, 0));
-        if (occ < 1) occ = 1;
-        occ_dev = dev;
-    }
-    const int sms = sm_count();
-    MOVAE_REQUIRE(sms > 0, MOVAE_ERR_CUDA, "CUDA device query failed (no GPU?)");
-    const int64_t n_items = P / (VEC ? 4 : 1);
     const int64_t tile_items = (int64_t)kGramThreads * U;
-    int64_t n_tiles = (n_items + tile_items - 1) / tile_items;
-    if (n_tiles < 1) n_tiles = 1;
-    int64_t grid = (int64_t)sms * occ;
-    if (grid > n_tiles) grid = n_tiles;
-    if (grid > kGramMaxBlocks) grid = kGramMaxBlocks;
-    unsigned int* counter = reinterpret_cast<unsigned int*>(ws);
-    double* partials = reinterpret_cast<double*>(reinterpret_cast<char*>(ws) + kGramHeaderBytes);
-    kern<<<(unsigned)grid, kGramThreads, 0, st>>>(J, P, ldJ, partials, counter, G, accumulate);
+    unsigned int grid = 0;
+    const int rc = persistent_grid<gram_kernel<K, U, VEC, MINB>>(kGramThreads, (P / (VEC ? 4 : 1) + tile_items - 1) / tile_items,
+                                                                 kGramMaxBlocks, &grid);
+    if (rc != MOVAE_OK) return rc;
+    const GramWorkspace w(ws);
+    gram_kernel<K, U, VEC, MINB><<<grid, kGramThreads, 0, st>>>(J, P, ldJ, w.partials, w.ticket, G, accumulate);
     MOVAE_CUDA_TRY(cudaGetLastError());
     return MOVAE_OK;
-}
-
-template <int K>
-static int dispatch_gram(const float* J, int64_t P, int64_t ldJ, double* G, int accumulate, void* ws, cudaStream_t st) {
-    const bool vec = (reinterpret_cast<uintptr_t>(J) % 16 == 0) && (ldJ % 4 == 0 || K == 1);
-    // registers: float64 accumulators cost 2*K(K+1)/2; small k affords deeper unroll and 2+ CTAs/SM
-    if (vec) {
-        if constexpr (K <= 2) return launch_gram<K, 8, true, 2>(J, P, ldJ, G, accumulate, ws, st);
-        else if constexpr (K <= 4) return launch_gram<K, 4, true, 2>(J, P, ldJ, G, accumulate, ws, st);
-        else return launch_gram<K, 2, true, 1>(J, P, ldJ, G, accumulate, ws, st);
-    } else {
-        if constexpr (K <= 4) return launch_gram<K, 8, false, 2>(J, P, ldJ, G, accumulate, ws, st);
-        else return launch_gram<K, 4, false, 1>(J, P, ldJ, G, accumulate, ws, st);
-    }
 }
 
 }  // namespace movae
@@ -102,16 +74,19 @@ static int gram_entry(const float* d_J, int k, int64_t P, int64_t ldJ, double* d
                   "gram: workspace too small (%zu < %zu)", ws_bytes, movae_gram_workspace_bytes(k));
     MOVAE_REQUIRE(reinterpret_cast<uintptr_t>(d_ws) % 8 == 0, MOVAE_ERR_WORKSPACE, "gram: workspace must be 8-byte aligned");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    switch (k) {
-        case 1: return dispatch_gram<1>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
-        case 2: return dispatch_gram<2>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
-        case 3: return dispatch_gram<3>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
-        case 4: return dispatch_gram<4>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
-        case 5: return dispatch_gram<5>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
-        case 6: return dispatch_gram<6>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
-        case 7: return dispatch_gram<7>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
-        default: return dispatch_gram<8>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
-    }
+    const bool vec = (reinterpret_cast<uintptr_t>(d_J) % 16 == 0) && (ldJ % 4 == 0 || k == 1);
+    // registers: float64 accumulators cost 2*K(K+1)/2; small k affords deeper unroll and 2+ CTAs/SM
+    return dispatch_k(k, [&](auto kc) {
+        constexpr int K = decltype(kc)::value;
+        if (vec) {
+            if constexpr (K <= 2) return launch_gram<K, 8, true, 2>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
+            else if constexpr (K <= 4) return launch_gram<K, 4, true, 2>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
+            else return launch_gram<K, 2, true, 1>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
+        } else {
+            if constexpr (K <= 4) return launch_gram<K, 8, false, 2>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
+            else return launch_gram<K, 4, false, 1>(d_J, P, ldJ, d_G, accumulate, d_ws, st);
+        }
+    });
 }
 
 int movae_gram_f32(const float* d_J, int k, int64_t P, int64_t ldJ, double* d_G, int accumulate, void* d_ws,

@@ -19,6 +19,35 @@ constexpr int kGramMaxBlocks = 2048;
 constexpr int kGramHeaderBytes = 256;
 constexpr int kGramChain = 64;   // float32 FMA chain length (columns) between promotions to float64
 
+// The workspace (movae_gram_workspace_bytes): a header, then one float64 partial per CTA from kGramHeaderBytes on.  Header:
+// byte 0 the ticket of the Gramian pass; the fused launches (aggregate.cu) also keep their exit counter at 4, their ready
+// flag at 128 and the six timestamps of their last launch at 192.
+struct GramWorkspace {
+    static constexpr int kTicket = 0, kExit = 4, kReady = 128, kStamps = 192;
+    unsigned int* ticket;
+    unsigned int* exit;
+    unsigned int* ready;
+    unsigned long long* stamps;
+    double* partials;
+    __host__ __device__ explicit GramWorkspace(void* ws) {
+        unsigned char* b = static_cast<unsigned char*>(ws);
+        ticket = reinterpret_cast<unsigned int*>(b + kTicket);
+        exit = reinterpret_cast<unsigned int*>(b + kExit);
+        ready = reinterpret_cast<unsigned int*>(b + kReady);
+        stamps = reinterpret_cast<unsigned long long*>(b + kStamps);
+        partials = reinterpret_cast<double*>(b + kGramHeaderBytes);
+    }
+};
+static_assert(GramWorkspace::kStamps + 6 * 8 <= kGramHeaderBytes, "the timestamps fit the header");
+
+// Row addressing of the tile helpers: row(i) is the first column of row i.  A flat J has its rows ldJ floats apart; the
+// segmented kernel's rows are separate tensors (aggregate.cu).
+struct FlatRows {
+    const float* J;
+    int64_t ldJ;
+    __device__ __forceinline__ const float* row(int i) const { return J + i * ldJ; }
+};
+
 template <int K>
 struct GramAcc {
     static constexpr int N = K * (K + 1) / 2;
@@ -65,9 +94,9 @@ struct PlainSteps {
 };
 
 // One tile of the Gramian pass: items [t0, t0 + tile) clipped to [t0, hi).
-template <int K, int U, bool VEC, class IO = PlainTileIO>
-__device__ __forceinline__ void gram_tile(const float* __restrict__ J, int64_t ldJ, int64_t t0, int64_t hi, bool full,
-                                          float (&acc)[GramAcc<K>::N], IO io = {}) {
+template <int K, int U, bool VEC, class Rows, class IO = PlainTileIO>
+__device__ __forceinline__ void gram_tile(const Rows& rows, int64_t t0, int64_t hi, bool full, float (&acc)[GramAcc<K>::N],
+                                          IO io = {}) {
     const int64_t base = t0 + threadIdx.x;
     if constexpr (VEC) {
         float4 v[K][U];
@@ -76,15 +105,14 @@ __device__ __forceinline__ void gram_tile(const float* __restrict__ J, int64_t l
             for (int i = 0; i < K; ++i)
 #pragma unroll
                 for (int u = 0; u < U; ++u)
-                    v[i][u] = io.load(reinterpret_cast<const float4*>(J + i * ldJ) + base + u * kGramThreads);
+                    v[i][u] = io.load(reinterpret_cast<const float4*>(rows.row(i)) + base + u * kGramThreads);
         } else {
 #pragma unroll
             for (int i = 0; i < K; ++i)
 #pragma unroll
                 for (int u = 0; u < U; ++u) {
                     const int64_t idx = base + u * kGramThreads;
-                    v[i][u] = idx < hi ? io.load(reinterpret_cast<const float4*>(J + i * ldJ) + idx)
-                                       : make_float4(0.f, 0.f, 0.f, 0.f);
+                    v[i][u] = idx < hi ? io.load(reinterpret_cast<const float4*>(rows.row(i)) + idx) : make_float4(0.f, 0.f, 0.f, 0.f);
                 }
         }
 #pragma unroll
@@ -110,7 +138,7 @@ __device__ __forceinline__ void gram_tile(const float* __restrict__ J, int64_t l
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const int64_t idx = base + u * kGramThreads;
-                v[i][u] = idx < hi ? io.load(J + i * ldJ + idx) : 0.f;
+                v[i][u] = idx < hi ? io.load(rows.row(i) + idx) : 0.f;
             }
 #pragma unroll
         for (int u = 0; u < U; ++u) {
@@ -120,6 +148,21 @@ __device__ __forceinline__ void gram_tile(const float* __restrict__ J, int64_t l
             gram_fma<K>(acc, x);
         }
     }
+}
+
+// Column c of the rows (a ragged tail of the float4 path) as a float32 chain of its own, promoted into acc64.
+template <int K, class Rows>
+__device__ __forceinline__ void gram_column(const Rows& rows, int64_t c, double (&acc64)[GramAcc<K>::N]) {
+    constexpr int NACC = GramAcc<K>::N;
+    float x[K];
+    float acc[NACC];
+#pragma unroll
+    for (int a = 0; a < NACC; ++a) acc[a] = 0.f;
+#pragma unroll
+    for (int i = 0; i < K; ++i) x[i] = rows.row(i)[c];
+    gram_fma<K>(acc, x);
+#pragma unroll
+    for (int a = 0; a < NACC; ++a) acc64[a] += (double)acc[a];
 }
 
 // Streams this CTA's share of J front to back (rr_schedule over gridDim.x CTAs) and adds the products into acc64.
@@ -135,6 +178,7 @@ __device__ __forceinline__ void gram_stream_tiles(const float* __restrict__ J, i
     constexpr int64_t tile_items = (int64_t)kGramThreads * U;
     const RRSchedule sch = rr_schedule(n_items, tile_items, blockIdx.x, gridDim.x);
     const int64_t n_steps = sch.rounds + (sch.rem_hi > sch.rem_lo ? 1 : 0);
+    const FlatRows rows{J, ldJ};
 
     int64_t r = 0;
     while (r < sch.rounds) {
@@ -144,7 +188,7 @@ __device__ __forceinline__ void gram_stream_tiles(const float* __restrict__ J, i
 #pragma unroll 1
         for (int f = 0; f < FLUSH && r < sch.rounds; ++f, ++r) {
             const int64_t t0 = (r * gridDim.x + blockIdx.x) * tile_items;
-            gram_tile<K, U, VEC>(J, ldJ, t0, t0 + tile_items, true, acc, steps(n_steps - 1 - r));
+            gram_tile<K, U, VEC>(rows, t0, t0 + tile_items, true, acc, steps(n_steps - 1 - r));
         }
 #pragma unroll
         for (int a = 0; a < NACC; ++a) acc64[a] += (double)acc[a];
@@ -153,23 +197,13 @@ __device__ __forceinline__ void gram_stream_tiles(const float* __restrict__ J, i
         float acc[NACC];
 #pragma unroll
         for (int a = 0; a < NACC; ++a) acc[a] = 0.f;
-        gram_tile<K, U, VEC>(J, ldJ, sch.rem_lo, sch.rem_hi, false, acc, steps(0));
+        gram_tile<K, U, VEC>(rows, sch.rem_lo, sch.rem_hi, false, acc, steps(0));
 #pragma unroll
         for (int a = 0; a < NACC; ++a) acc64[a] += (double)acc[a];
     }
 
     // ragged tail of the float4 path: columns 4*(P/4) .. P-1, one thread each in CTA 0
-    if (VEC && blockIdx.x == 0 && tid < (int)(P - n_items * W)) {
-        float x[K];
-        float acc[NACC];
-#pragma unroll
-        for (int a = 0; a < NACC; ++a) acc[a] = 0.f;
-#pragma unroll
-        for (int i = 0; i < K; ++i) x[i] = J[i * ldJ + n_items * W + tid];
-        gram_fma<K>(acc, x);
-#pragma unroll
-        for (int a = 0; a < NACC; ++a) acc64[a] += (double)acc[a];
-    }
+    if (VEC && blockIdx.x == 0 && tid < (int)(P - n_items * W)) gram_column<K>(rows, n_items * W + tid, acc64);
 }
 
 // CTA reduce (shuffle within warps, fixed-order sum across the 8 warps), store this CTA's partial, take a

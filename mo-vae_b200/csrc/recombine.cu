@@ -22,40 +22,14 @@ recombine_kernel(const float* __restrict__ J, int64_t P, int64_t ldJ, const floa
 template <int K, int U, bool VEC>
 static int launch_recombine(const float* J, int64_t P, int64_t ldJ, const float* w, float* out, int accumulate,
                             cudaStream_t st) {
-    auto kern = recombine_kernel<K, U, VEC>;
-    static thread_local int occ_dev = -1, occ = 0;      // cached per (host thread, device)
-    int dev = 0;
-    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-    if (occ_dev != dev) {
-        MOVAE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kRecThreads, 0));
-        if (occ < 1) occ = 1;
-        occ_dev = dev;
-    }
-    const int sms = sm_count();
-    MOVAE_REQUIRE(sms > 0, MOVAE_ERR_CUDA, "CUDA device query failed (no GPU?)");
-    const int64_t n_items = P / (VEC ? 4 : 1);
     const int64_t tile_items = (int64_t)kRecThreads * U;
-    int64_t n_tiles = (n_items + tile_items - 1) / tile_items;
-    if (n_tiles < 1) n_tiles = 1;
-    int64_t grid = (int64_t)sms * occ;
-    if (grid > n_tiles) grid = n_tiles;
-    kern<<<(unsigned)grid, kRecThreads, 0, st>>>(J, P, ldJ, w, out, accumulate);
+    unsigned int grid = 0;
+    const int rc = persistent_grid<recombine_kernel<K, U, VEC>>(kRecThreads, (P / (VEC ? 4 : 1) + tile_items - 1) / tile_items,
+                                                                INT64_MAX, &grid);
+    if (rc != MOVAE_OK) return rc;
+    recombine_kernel<K, U, VEC><<<grid, kRecThreads, 0, st>>>(J, P, ldJ, w, out, accumulate);
     MOVAE_CUDA_TRY(cudaGetLastError());
     return MOVAE_OK;
-}
-
-template <int K>
-static int dispatch_recombine(const float* J, int64_t P, int64_t ldJ, const float* w, float* out, int accumulate,
-                              cudaStream_t st) {
-    const bool vec = (reinterpret_cast<uintptr_t>(J) % 16 == 0) && (reinterpret_cast<uintptr_t>(out) % 16 == 0) &&
-                     (ldJ % 4 == 0 || K == 1);
-    if (vec) {
-        if constexpr (K <= 4) return launch_recombine<K, 4, true>(J, P, ldJ, w, out, accumulate, st);
-        else return launch_recombine<K, 2, true>(J, P, ldJ, w, out, accumulate, st);
-    } else {
-        if constexpr (K <= 4) return launch_recombine<K, 8, false>(J, P, ldJ, w, out, accumulate, st);
-        else return launch_recombine<K, 4, false>(J, P, ldJ, w, out, accumulate, st);
-    }
 }
 
 }  // namespace movae
@@ -69,14 +43,16 @@ extern "C" int movae_recombine_f32(const float* d_J, int k, int64_t P, int64_t l
     if (P == 0) return MOVAE_OK;
     MOVAE_REQUIRE(d_J && d_w && d_grad, MOVAE_ERR_INVALID, "recombine: null pointer");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    switch (k) {
-        case 1: return dispatch_recombine<1>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
-        case 2: return dispatch_recombine<2>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
-        case 3: return dispatch_recombine<3>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
-        case 4: return dispatch_recombine<4>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
-        case 5: return dispatch_recombine<5>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
-        case 6: return dispatch_recombine<6>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
-        case 7: return dispatch_recombine<7>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
-        default: return dispatch_recombine<8>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
-    }
+    const bool vec = (reinterpret_cast<uintptr_t>(d_J) % 16 == 0) && (reinterpret_cast<uintptr_t>(d_grad) % 16 == 0) &&
+                     (ldJ % 4 == 0 || k == 1);
+    return dispatch_k(k, [&](auto kc) {
+        constexpr int K = decltype(kc)::value;
+        if (vec) {
+            if constexpr (K <= 4) return launch_recombine<K, 4, true>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
+            else return launch_recombine<K, 2, true>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
+        } else {
+            if constexpr (K <= 4) return launch_recombine<K, 8, false>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
+            else return launch_recombine<K, 4, false>(d_J, P, ldJ, d_w, d_grad, accumulate, st);
+        }
+    });
 }

@@ -41,6 +41,22 @@ def test_workspace_query_is_host_only():
     assert lib.movae_gram_workspace_bytes(8) > lib.movae_gram_workspace_bytes(3)
 
 
+def test_fused_segment_launch_rejects_a_misaligned_workspace():
+    import movae_b200
+    from movae_b200 import _lib
+
+    lib = movae_b200.lib()
+    segs = _lib.JacSegments(n_segments=1, k=1)
+    segs.n[0] = 4
+    segs.rows[0][0] = 0x10000                                          # never dereferenced: validation fails first
+    spec = _lib.SolveSpec(kind=_lib.SOLVE_CONSTANT)
+    ws_bytes = lib.movae_gram_workspace_bytes(1)
+    rc = lib.movae_aggregate_segments_f32(ctypes.byref(segs), ctypes.byref(spec), None, None, None, 0, 0x20000, None, None,
+                                          0x30004, ws_bytes, None, None)
+    assert rc == 4, lib.movae_last_error()                            # MOVAE_ERR_WORKSPACE
+    assert b"8-byte aligned" in lib.movae_last_error()
+
+
 def test_optimizer_and_extraction_host_side_contracts():
     import ctypes
 

@@ -173,7 +173,8 @@ def test_status_is_checkable_on_every_weighting(mv):
 @pytest.mark.parametrize("name", ["upgrad", "aligned_mtl", "mgda_lgn", "comfort"])
 def test_segmented_launch_equals_the_flat_jacobian(mv, oa, k, name):
     """movae_aggregate_segments_f32: the rows are separate tensors per segment (odd sizes, ragged tails, one tile-crossing
-    segment, an identically zero row through a shared zero buffer) -- same Gramian, weights and gradient as the flat J."""
+    segment, an identically zero row through a shared zero buffer) -- same Gramian, weights and gradient as the flat J, and
+    bit for bit the gradient K3 computes from the same weights on J laid out like `out`."""
     sizes = [27, 4, 1, 130, 65_537, 300_000, 8, 1_048_576 + 3]
     g = torch.Generator(device="cuda").manual_seed(17 + k)
     scale = torch.logspace(0, -1, k, device="cuda")
@@ -185,6 +186,9 @@ def test_segmented_launch_equals_the_flat_jacobian(mv, oa, k, name):
         offs.append(off)
         off += (n + 3) // 4 * 4
     J = torch.cat([torch.stack([rows[i][s][:n] for i in range(k)]) for s, n in enumerate(sizes)], dim=1).contiguous()
+    J_padded = torch.zeros(k, off, device="cuda")                   # each segment at its offset in `out`, zero columns between
+    for s, (o, n) in enumerate(zip(offs, sizes)):
+        J_padded[:, o:o + n] = torch.stack([rows[i][s][:n] for i in range(k)])
     losses = torch.tensor([LOSSES[i % 5] for i in range(k)], device="cuda")
 
     def make():
@@ -209,10 +213,12 @@ def test_segmented_launch_equals_the_flat_jacobian(mv, oa, k, name):
     for o, n in zip(offs, sizes):
         pad[o:o + n] = False
     assert bool((out[pad] == 5.0).all())                     # padding columns are never written
+    assert torch.equal(out[~pad], mv.ops.recombine(J_padded, w)[~pad])
     before = out.clone()
-    agg.aggregate_segments_into(rows, sizes, offs, out, accumulate=True)
+    w2 = agg.aggregate_segments_into(rows, sizes, offs, out, accumulate=True)
     got2 = torch.cat([out[o:o + n] for o, n in zip(offs, sizes)])
     np.testing.assert_allclose(got2.cpu().numpy(), 2.0 * torch.cat([before[o:o + n] for o, n in zip(offs, sizes)]).cpu().numpy(), rtol=1e-6, atol=1e-7)
+    assert torch.equal(out[~pad], mv.ops.recombine(J_padded, w2, out=before.clone(), accumulate=True)[~pad])
 
 
 class _TinyNet(torch.nn.Module):
