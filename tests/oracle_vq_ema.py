@@ -32,6 +32,15 @@ def ema_update_fp64(flat: torch.Tensor, idx: torch.Tensor, cluster_size: torch.T
     idx = idx.to(torch.int64)
     count = torch.bincount(idx, minlength=K).to(torch.float64) * count_scale
     S = torch.zeros(K, z.shape[1], dtype=torch.float64).index_add_(0, idx, z) * count_scale
+    return ema_update_from_stats(count, S, cluster_size, embed_avg, decay, eps)
+
+
+def ema_update_from_stats(count: torch.Tensor, S: torch.Tensor, cluster_size: torch.Tensor, embed_avg: torch.Tensor, decay: float,
+                          eps: float) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The same update from the batch statistics count [K] and S [K, D], on their device (for batches whose rows are
+    too many to gather in one float64 tensor)."""
+    K = cluster_size.shape[0]
+    count, S = count.to(torch.float64), S.to(torch.float64)
     cs = decay * cluster_size.to(torch.float64) + (1 - decay) * count
     ea = decay * embed_avg.to(torch.float64) + (1 - decay) * S
     n = cs.sum()
