@@ -52,6 +52,20 @@ int persistent_grid(int threads, int64_t n_tiles, int64_t cap, unsigned int* gri
     return MOVAE_OK;
 }
 
+// Lets `kern` launch with `bytes` of dynamic shared memory (more than 48 KB needs this opt-in).  The attribute belongs to
+// the device current when it is set, so it is set once per kernel instantiation, host thread and device, as above.
+template <auto kern>
+int allow_dynamic_smem(int bytes) {
+    static thread_local int attr_dev = -1;
+    int dev = 0;
+    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
+    if (attr_dev != dev) {
+        MOVAE_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+        attr_dev = dev;
+    }
+    return MOVAE_OK;
+}
+
 // Returns f(std::integral_constant<int, K>{}) for K = k; k is 1 .. MOVAE_MAX_K (larger k take MOVAE_MAX_K).
 template <int K = 1, class F>
 int dispatch_k(int k, F&& f) {

@@ -4,28 +4,6 @@
 
 namespace movae {
 
-// launchers defined in vq_argmin_tc.cu / vq_argmin_exact.cu / vq_gather.cu / vq_backward.cu
-int launch_vq_argmin_tc(const float* z, int64_t N, int64_t HW, const float* E, long long* idx, unsigned int* ws_words, float* dbg,
-                        cudaStream_t st);
-int launch_vq_argmin_exact(const float* z, int64_t N, int D, int64_t HW, const float* E, int K, long long* idx, cudaStream_t st);
-int launch_vq_gather(const float* z, int64_t N, int D, int64_t HW, const float* E, int K, const long long* idx,
-                     float* q_out, float* loss_out, int* usage_out, unsigned char* ws, cudaStream_t st);
-int launch_vq_usage(const long long* idx, int64_t n, int K, int* usage_out, unsigned char* ws, cudaStream_t st);
-int launch_vq_backward(const float* grad_out, const float* g_commit, const float* g_embed, const float* z, int64_t N, int D,
-                       int64_t HW, const float* E, int K, const long long* idx, float* dz, float* dE, float* partials,
-                       cudaStream_t st);
-int launch_vq_pack_codes(const long long* idx, int64_t n, int K, void* out, int code_bytes, unsigned int* bitmap, cudaStream_t st);
-int launch_vq_bitmap_count(const unsigned int* bitmap, int K, int* count, cudaStream_t st);
-int vq_backward_parts(int64_t n_rows, int K, int D);
-size_t vq_backward_part_bytes();
-size_t vq_ema_workspace_bytes(int64_t n_rows, int K, int D);
-int launch_vq_ema_stats(const float* z, int64_t N, int D, int64_t HW, const long long* idx, int K, float* stats, unsigned char* ws,
-                        cudaStream_t st);
-int launch_vq_ema_apply(const float* stats, int K, int D, double decay, double eps, float* E, float* cluster_size, float* embed_avg,
-                        float* E_prev, unsigned char* ws, cudaStream_t st);
-int launch_vq_ema_update(const float* z, int64_t N, int D, int64_t HW, const long long* idx, int K, double decay, double eps, float* E,
-                         float* cluster_size, float* embed_avg, float* E_prev, unsigned char* ws, cudaStream_t st);
-
 constexpr size_t kVqWsListOff = kWsListOff;
 constexpr int kVqMaxK = 65536;
 
@@ -109,7 +87,7 @@ int movae_vq_forward_f32(const float* d_z, int64_t B, int D, int64_t HW, const f
 
 size_t movae_vq_backward_workspace_bytes(int64_t n_rows, int K, int D) {
     if (n_rows < 0 || K < 1 || D < 1) return 0;
-    return (size_t)movae::vq_backward_parts(n_rows, K, D) * movae::vq_backward_part_bytes();
+    return (size_t)movae::vq_backward_parts(n_rows, K, D) * movae::kPartFloats * sizeof(float);
 }
 
 int movae_vq_backward_f32(const float* d_grad_quantized, const float* d_g_commit, const float* d_g_embed, const float* d_z,

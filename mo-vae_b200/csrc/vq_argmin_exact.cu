@@ -253,14 +253,9 @@ int launch_vq_argmin_exact(const float* z, int64_t N, int D, int64_t HW, const f
     const int64_t cap = stage ? (int64_t)sms : (int64_t)sms * 4;
     if (grid > cap) grid = cap;
     if (grid < 1) grid = 1;
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-    if (configured_dev != dev) {
-        MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_argmin_exact_kernel<true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kExMaxSmem));
-        MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_argmin_exact_kernel<false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kExMaxSmem));
-        configured_dev = dev;
-    }
+    const int rc = stage ? allow_dynamic_smem<vq_argmin_exact_kernel<true, 4>>((int)kExMaxSmem)
+                         : allow_dynamic_smem<vq_argmin_exact_kernel<false, 1>>((int)kExMaxSmem);
+    if (rc != MOVAE_OK) return rc;
     if (stage)
         vq_argmin_exact_kernel<true, 4><<<(unsigned)grid, kExThreads, staged, st>>>(z, N, D, HW, E, K, list, list_count, idx);
     else

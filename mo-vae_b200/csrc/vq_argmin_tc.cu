@@ -612,14 +612,9 @@ vq_argmin_tc_kernel(const float* __restrict__ z, int64_t N, int64_t HW, const fl
 // Host launcher (called from vq_api.cu).  `ws_words`: the head of the (zero-initialised) quantizer workspace.
 int launch_vq_argmin_tc(const float* z, int64_t N, int64_t HW, const float* E, long long* idx, unsigned int* ws_words,
                         float* dbg, cudaStream_t st) {
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-    if (configured_dev != dev) {
-        MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_argmin_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmemBytes));
-        MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_argmin_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmemBytes));
-        configured_dev = dev;
-    }
+    const int rc = dbg == nullptr ? allow_dynamic_smem<vq_argmin_tc_kernel<false>>((int)kTcSmemBytes)
+                                  : allow_dynamic_smem<vq_argmin_tc_kernel<true>>((int)kTcSmemBytes);
+    if (rc != MOVAE_OK) return rc;
     const int sms = sm_count();
     MOVAE_REQUIRE(sms > 0, MOVAE_ERR_CUDA, "CUDA device query failed (no GPU?)");
     const int64_t n_tiles = (N + kTcTileM - 1) / kTcTileM;

@@ -64,7 +64,7 @@ vq_backward_atomic_kernel(const float* __restrict__ grad_out, const float* __res
 // with REGISTER accumulators selected by a warp-uniform switch (a 5-level compare-and-branch tree per row, 427
 // instructions per warp and tile, 41% of the stall samples at the per-tile barrier, 4-way conflicts on the TMA-written
 // [channel][row] tile) 0.63-0.69 ms = 25% of HBM peak.
-constexpr int kBwK = 512, kBwD = 64, kBwRows = 128, kBwThreads = 1024, kBwChunks = kBwRows / 32;
+constexpr int kBwRows = kPartTileRows, kBwThreads = 1024, kBwChunks = kBwRows / 32;
 constexpr int kBwParts = kBwThreads / kBwRows;                 // copy roles per row: each covers kBwD / kBwParts channels
 constexpr int kBwOwn = kBwK / (kBwThreads / 32);               // codes owned by one warp (16)
 constexpr int kBwOwnShift = 4;
@@ -74,7 +74,6 @@ constexpr int kBwDepth = 3;              // tile buffers: two tiles (64 KB) in f
 constexpr size_t kBwSmemBytes = sizeof(float) * ((size_t)kBwK * kBwD + kBwDepth * (size_t)kBwRows * kBwLdRow) +
                                 sizeof(unsigned short) * (kBwDepth * (size_t)kBwRows);
 static_assert(kBwSmemBytes <= 227 * 1024, "K6b shared memory");
-constexpr size_t kBwPartFloats = (size_t)kBwK * kBwD + kBwK;      // per-CTA partial: S [K, D] then counts [K] (as int bits)
 constexpr int kDzThreads = 512;
 
 template <bool STAGE, int THREADS>
@@ -215,7 +214,7 @@ vq_backward_dE_kernel(const float* __restrict__ z, int64_t N, int64_t HW, const 
     }
     asm volatile("cp.async.wait_group 0;" ::: "memory");
     __syncthreads();
-    float* out = partials + (size_t)blockIdx.x * kBwPartFloats;
+    float* out = partials + (size_t)blockIdx.x * kPartFloats;
     for (int i = tid; i < kBwK * kBwD; i += kBwThreads) out[i] = S[i];
     if (lane < kBwOwn) out[kBwK * kBwD + warp * kBwOwn + lane] = __int_as_float(my_count);   // lane l of warp w counts code 16 w + l
 }
@@ -274,26 +273,10 @@ __device__ __forceinline__ void tma_box_3d(void* smem_dst, const CUtensorMap* tm
         "l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1), "r"(c2), "r"((uint32_t)__cvta_generic_to_shared(bar))
         : "memory");
 }
-__device__ __forceinline__ void mbar_init_(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(count) : "memory");
-}
 __device__ __forceinline__ void mbar_expect_tx_(uint64_t* bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(bytes)
                  : "memory");
 }
-__device__ __forceinline__ void mbar_arrive_(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"((uint32_t)__cvta_generic_to_shared(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_(uint64_t* bar, uint32_t parity) {
-    uint32_t ok = 0;
-    while (!ok)
-        asm volatile(
-            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(parity)
-            : "memory");
-}
-
 __device__ __forceinline__ int tm_owner(int code) { return (code * kTmConsumers) >> 9; }   // owner warp of a code: 18 or 19 codes each
 __device__ __forceinline__ int tm_first(int w) { return (w * kBwK + kTmConsumers - 1) / kTmConsumers; }   // first code of owner w
 // TMEM as a 256 KB scratchpad: lane l of the issuing warp reads / writes two consecutive 32-bit columns of TMEM lane
@@ -330,11 +313,11 @@ vq_backward_dE_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t N, i
     if (tid < kBwK) cnt[tid] = 0;
     if (tid == 0) {
         for (int b = 0; b < kTmDepth; ++b) {
-            mbar_init_(&full[b], 1);
-            mbar_init_(&routed[b], 1);
-            mbar_init_(&empty[b], kTmConsumers);
+            tc::mbar_init(&full[b], 1);
+            tc::mbar_init(&routed[b], 1);
+            tc::mbar_init(&empty[b], kTmConsumers);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        tc::mbar_fence_init();
     }
     if (warp == 31) tc::tmem_alloc(tmem_slot, 512);                                // the per-code sums S live in TENSOR MEMORY
     tc::tc_fence_before_sync();
@@ -351,7 +334,7 @@ vq_backward_dE_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t N, i
             for (int64_t unit = blockIdx.x; unit < n_units; unit += gridDim.x, ++it) {
                 const int buf = (int)(it % kTmDepth);
                 uint8_t* ub = units + buf * kTmUnitBytes;
-                mbar_wait_(&empty[buf], ((it / kTmDepth) & 1u) ^ 1u);       // a fresh barrier passes parity 1
+                tc::mbar_wait(&empty[buf], ((it / kTmDepth) & 1u) ^ 1u);   // a fresh barrier passes parity 1
                 const uint32_t n0 = (uint32_t)(unit * kTmRows);
                 const int rows = (int)((N - n0) < kTmRows ? (N - n0) : kTmRows);      // a multiple of 32 (N % 32 == 0)
                 mbar_expect_tx_(&full[buf], (uint32_t)(rows / 32) * kTmChunkBytes + (uint32_t)rows * 8u);
@@ -379,7 +362,7 @@ vq_backward_dE_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t N, i
             unsigned int* order = sz + kTmChunks * 32;
             const int64_t n0 = unit * kTmRows;
             const int rows = (int)((N - n0) < kTmRows ? (N - n0) : kTmRows);
-            mbar_wait_(&full[buf], (it / kTmDepth) & 1u);
+            tc::mbar_wait(&full[buf], (it / kTmDepth) & 1u);
             // (the owners are done with this buffer's route block: the producer refilled it only after empty[buf])
 #pragma unroll
             for (int q = 0; q < kTmChunks; ++q) sz[q * 32 + lane] = 0u;
@@ -427,7 +410,7 @@ vq_backward_dE_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t N, i
                     order[base + rank[q]] = ((((uint32_t)q << 13) | row_off) << 5) | (uint32_t)(code[q] - tm_first(owner[q]));
             }
             __syncwarp();
-            if (lane == 0) mbar_arrive_(&routed[buf]);                   // release: start and order are visible to waiters
+            if (lane == 0) tc::mbar_arrive(&routed[buf]);               // release: start and order are visible to waiters
         }
     } else {
         // ---- owner warps: warp w owns the codes c with tm_owner(c) == w; lane l adds channels l and l + 32.  The sums live in
@@ -444,8 +427,8 @@ vq_backward_dE_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t N, i
             const unsigned int* start = reinterpret_cast<const unsigned int*>(routes + buf * kTmRouteBytes);
             const unsigned int* order = start + 32 + kTmChunks * 32;
             const uint32_t par = (it / kTmDepth) & 1u;
-            mbar_wait_(&routed[buf], par);
-            mbar_wait_(&full[buf], par);                                 // already complete: makes the TMA writes visible here too
+            tc::mbar_wait(&routed[buf], par);
+            tc::mbar_wait(&full[buf], par);                             // already complete: makes the TMA writes visible here too
             unsigned i = start[warp];
             const unsigned i_end = start[warp + 1];
             if (i < i_end) {
@@ -471,9 +454,9 @@ vq_backward_dE_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t N, i
                 }
             }
             __syncwarp();
-            if (lane == 0) mbar_arrive_(&empty[buf]);
+            if (lane == 0) tc::mbar_arrive(&empty[buf]);
         }
-        float* out_w = partials + (size_t)blockIdx.x * kBwPartFloats + (size_t)first * kBwD + lane;
+        float* out_w = partials + (size_t)blockIdx.x * kPartFloats + (size_t)first * kBwD + lane;
         for (int j = 0; j < n_own; ++j) {
             float s0, s1;
             tmem_ld_x2(tbase + 2u * (uint32_t)j, s0, s1);
@@ -487,7 +470,7 @@ vq_backward_dE_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t N, i
         tc::tc_fence_after_sync();
         tc::tmem_dealloc(tmem_base, 512);
     }
-    float* out = partials + (size_t)blockIdx.x * kBwPartFloats;
+    float* out = partials + (size_t)blockIdx.x * kPartFloats;
     if (tid < kBwK) out[kBwK * kBwD + tid] = __int_as_float(cnt[tid]);
 }
 
@@ -517,76 +500,30 @@ static int make_z_tensor_map(const float* z, int64_t B, int64_t HW, CUtensorMap*
     return MOVAE_OK;
 }
 
-// dE[j, d] += g_embed * 2 / (N D) * (count_j e[j, d] - S[j, d]).  Per-CTA partials combined in float64 in a FIXED order:
-// thread (q, g) of a CTA sums the partials p = g, g + 4, g + 8, ... of output quad q (16-byte loads, 4 in flight), then the
-// four group sums are added in the order g = 0, 1, 2, 3 -- bit-reproducible, and 16 partial loads in flight per output
-// quad instead of 8 scalar ones per output element (the reduction of 148 partials was a 26 us latency chain).
-// ema_combine_partials (vq_ema.cu) repeats this combine for VectorQuantizerEMA: keep the two identical.
-constexpr int kRdGroups = 4, kRdQuads = 64, kRdThreads = kRdGroups * kRdQuads;
+// dE[j, d] += g_embed * 2 / (N D) * (count_j e[j, d] - S[j, d]), with count_j and S_j combined from K6b's partials in
+// the fixed float64 order of k6b_combine_partials: bit-reproducible.
 __global__ void __launch_bounds__(kRdThreads)
 vq_dE_reduce_kernel(const float* __restrict__ partials, int n_parts, const float* __restrict__ g_embed,
                     const float* __restrict__ E, int64_t N, float* __restrict__ dE) {
-    __shared__ double sm_s[kRdGroups][kRdQuads][4];
-    __shared__ long long sm_c[kRdGroups][kRdQuads];
     const int q = threadIdx.x % kRdQuads, g = threadIdx.x / kRdQuads;
     const int quad = blockIdx.x * kRdQuads + q;                 // output elements 4 quad .. 4 quad + 3 (one code: D % 4 == 0)
-    const int j = quad * 4 / kBwD;
-    double s[4] = {0.0, 0.0, 0.0, 0.0};
-    long long c = 0;
-    if (quad < kBwK * kBwD / 4) {
-        for (int p0 = g; p0 < n_parts; p0 += kRdGroups * 4) {
-            float4 v[4];
-            int cv[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int p = p0 + u * kRdGroups;
-                const float* part = partials + (size_t)(p < n_parts ? p : 0) * kBwPartFloats;
-                v[u] = p < n_parts ? __ldcs(reinterpret_cast<const float4*>(part) + quad) : make_float4(0.f, 0.f, 0.f, 0.f);
-                cv[u] = p < n_parts ? __float_as_int(__ldg(part + kBwK * kBwD + j)) : 0;
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                s[0] += (double)v[u].x; s[1] += (double)v[u].y; s[2] += (double)v[u].z; s[3] += (double)v[u].w;
-                c += (long long)cv[u];
-            }
-        }
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) sm_s[g][q][i] = s[i];
-    sm_c[g][q] = c;
-    __syncthreads();
+    double st[4];
+    long long ct;
+    k6b_combine_partials(partials, n_parts, quad, q, g, st, ct);
     if (g == 0 && quad < kBwK * kBwD / 4) {
         const double ce = (double)__ldg(g_embed) * (double)(2.0f / (float)((double)N * (double)kBwD));
         const float4 e = __ldg(reinterpret_cast<const float4*>(E) + quad);
         const float ev[4] = {e.x, e.y, e.z, e.w};
         float4 out = reinterpret_cast<float4*>(dE)[quad];
         float* ov = reinterpret_cast<float*>(&out);
-        long long ct = 0;
 #pragma unroll
-        for (int gg = 0; gg < kRdGroups; ++gg) ct += sm_c[gg][q];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            double st = 0.0;
-#pragma unroll
-            for (int gg = 0; gg < kRdGroups; ++gg) st += sm_s[gg][q][i];
-            ov[i] += (float)(ce * ((double)ct * (double)ev[i] - st));
-        }
+        for (int i = 0; i < 4; ++i) ov[i] += (float)(ce * ((double)ct * (double)ev[i] - st[i]));
         reinterpret_cast<float4*>(dE)[quad] = out;
     }
 }
 
-// Number of per-CTA [K, D] partial buffers the segmented backward needs for n_rows (0 = generic path).
-size_t vq_backward_part_bytes() { return kBwPartFloats * sizeof(float); }
-
-int vq_backward_parts(int64_t n_rows, int K, int D) {
-    if (K != kBwK || D != kBwD || n_rows <= 0) return 0;
-    const int64_t tiles = (n_rows + kBwRows - 1) / kBwRows;
-    return (int)(tiles < 160 ? tiles : 160);
-}
-
-// K6b's per-CTA partials (S [K, D] then the counts, kBwPartFloats each) for K = 512, D = 64: the tensor-map kernel when
+// K6b's per-CTA partials (S [K, D] then the counts, kPartFloats each) for K = 512, D = 64: the tensor-map kernel when
 // 32-row boxes never straddle images and the copies are 16-byte aligned, else the cp.async one.  *n_parts = CTAs launched.
-// The caller has configured the kernels' dynamic shared memory on this device.
 int launch_k6b_partials(const float* z, int64_t N, int64_t HW, const long long* idx, float* partials, int* n_parts,
                         cudaStream_t st) {
     int grid = vq_backward_parts(N, kBwK, kBwD);
@@ -595,11 +532,15 @@ int launch_k6b_partials(const float* z, int64_t N, int64_t HW, const long long* 
                         HW * 4 * kBwD < ((int64_t)1 << 40);
     if (tma_ok) {
         CUtensorMap tmap;
-        const int rc = make_z_tensor_map(z, N / HW, HW, &tmap);
+        int rc = make_z_tensor_map(z, N / HW, HW, &tmap);
+        if (rc == MOVAE_OK) rc = allow_dynamic_smem<vq_backward_dE_tma_kernel>((int)kTmSmemBytes);
         if (rc != MOVAE_OK) return rc;
         vq_backward_dE_tma_kernel<<<grid, kTmThreads, kTmSmemBytes, st>>>(tmap, N, HW, idx, partials);
-    } else
+    } else {
+        const int rc = allow_dynamic_smem<vq_backward_dE_kernel>((int)kBwSmemBytes);
+        if (rc != MOVAE_OK) return rc;
         vq_backward_dE_kernel<<<grid, kBwThreads, kBwSmemBytes, st>>>(z, N, HW, idx, partials);
+    }
     MOVAE_CUDA_TRY(cudaGetLastError());
     *n_parts = grid;
     return MOVAE_OK;
@@ -613,19 +554,12 @@ int launch_vq_backward(const float* grad_out, const float* g_commit, const float
     const bool want_dE = dE != nullptr && g_embed != nullptr;
     const bool quads_ok = !want_dE || (reinterpret_cast<uintptr_t>(dE) % 16 == 0 && reinterpret_cast<uintptr_t>(E) % 16 == 0);
     if (K == kBwK && D == kBwD && (partials != nullptr || !want_dE) && quads_ok) {
-        static thread_local int configured_dev = -1;
-        int dev = 0;
-        MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-        if (configured_dev != dev) {
-            MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_backward_dE_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwSmemBytes));
-            MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_backward_dE_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTmSmemBytes));
-            MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_backward_dz_kernel<true, kDzThreads>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-            configured_dev = dev;
-        }
         if (dz != nullptr && N <= kSmallN) {
             vq_backward_dz_kernel<false, 256><<<(unsigned)((N + 255) / 256), 256, 0, st>>>(grad_out, g_commit, z, N, D, HW, E, K, idx, dz);
             MOVAE_CUDA_TRY(cudaGetLastError());
         } else if (dz != nullptr) {
+            const int rc = allow_dynamic_smem<vq_backward_dz_kernel<true, kDzThreads>>(160 * 1024);
+            if (rc != MOVAE_OK) return rc;
             int64_t grid = (N + kDzThreads - 1) / kDzThreads;
             if (grid > sms) grid = sms;
             vq_backward_dz_kernel<true, kDzThreads><<<(unsigned)grid, kDzThreads, (size_t)K * (D + 1) * sizeof(float), st>>>(
@@ -646,19 +580,6 @@ int launch_vq_backward(const float* grad_out, const float* g_commit, const float
     if (grid < 1) grid = 1;
     vq_backward_atomic_kernel<<<(unsigned)grid, 256, 0, st>>>(grad_out, g_commit, g_embed, z, N, D, HW, E, K, idx, dz, dE);
     MOVAE_CUDA_TRY(cudaGetLastError());
-    return MOVAE_OK;
-}
-
-// K6b's kernels need more than 48 KB of dynamic shared memory: configure them once per device (per host thread).
-int configure_k6b_partials() {
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-    if (configured_dev != dev) {
-        MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_backward_dE_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwSmemBytes));
-        MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_backward_dE_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTmSmemBytes));
-        configured_dev = dev;
-    }
     return MOVAE_OK;
 }
 

@@ -196,13 +196,8 @@ int launch_vq_gather(const float* z, int64_t N, int D, int64_t HW, const float* 
         return MOVAE_OK;
     }
     if (stage_bytes <= 160 * 1024) {
-        static thread_local int configured_dev = -1;
-        int dev = 0;
-        MOVAE_CUDA_TRY(cudaGetDevice(&dev));
-        if (configured_dev != dev) {
-            MOVAE_CUDA_TRY(cudaFuncSetAttribute(vq_gather_kernel<true, kGatherThreads>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-            configured_dev = dev;
-        }
+        const int rc = allow_dynamic_smem<vq_gather_kernel<true, kGatherThreads>>(160 * 1024);
+        if (rc != MOVAE_OK) return rc;
         vq_gather_kernel<true, kGatherThreads><<<(unsigned)grid, kGatherThreads, stage_bytes, st>>>(z, N, D, HW, E, K, idx, q_out,
                                                                                                  loss_out, usage_out, ws);
     } else {

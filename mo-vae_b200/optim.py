@@ -445,7 +445,7 @@ class GraphedStep:
         from . import autojac, ops as _ops, quantizer as _q
 
         self._keepalive = (list(autojac._J_CACHE.values()) + list(autojac._ZEROS.values()) + list(_ops._workspaces.values()) +
-                           list(_q._workspaces.values()) + list(_q._scratches.values()))
+                           list(_q._buffers.values()))
         self.replays = 0
 
     def __call__(self):

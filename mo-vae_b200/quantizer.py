@@ -19,33 +19,27 @@ from torch import Tensor, nn
 
 from . import _lib as L
 
-_workspaces: dict = {}
+_buffers: dict = {}
 
 
-def _workspace(device: torch.device, n_rows: int, K: int, D: int, stream: int) -> Tensor:
-    """One zero-initialised workspace per (device, stream); grown when a bigger batch shows up."""
+def _buffer(kind: str, device: torch.device, stream: int, nbytes: int, zero: bool = True) -> Tensor:
+    """The device buffer of `kind` for (device, stream), replaced by a bigger one when a call needs more bytes: "vq" (the
+    search / gather workspace), "ema" (the EMA update's workspace), "k6" (K6's per-CTA partials).  A workspace is
+    zero-filled when it is allocated and the kernels leave it clean; the K6 scratch (`zero=False`) is written before it
+    is read.  GraphedStep keeps every buffer of this cache alive for as long as a captured graph uses it."""
+    key = (kind, device.index, stream)
+    buf = _buffers.get(key)
+    if buf is None or buf.numel() < nbytes:
+        buf = (torch.zeros if zero else torch.empty)(nbytes, dtype=torch.uint8, device=device)
+        _buffers[key] = buf
+    return buf
+
+
+def _workspace_bytes(n_rows: int, K: int, D: int) -> int:
     need = L.lib().movae_vq_workspace_bytes(n_rows, K, D)
     if need == 0:
         raise RuntimeError(f"movae_b200: num_embeddings={K} is not supported by this CUDA build")
-    key = (device.index, stream)
-    ws = _workspaces.get(key)
-    if ws is None or ws.numel() < need:
-        ws = torch.zeros(need, dtype=torch.uint8, device=device)
-        _workspaces[key] = ws
-    return ws
-
-
-_scratches: dict = {}
-
-
-def _scratch(device: torch.device, nbytes: int, stream: int) -> Tensor:
-    """Uninitialised per-(device, stream) scratch for K6's per-CTA codebook-gradient partials."""
-    key = (device.index, stream)
-    buf = _scratches.get(key)
-    if buf is None or buf.numel() < nbytes:
-        buf = torch.empty(nbytes, dtype=torch.uint8, device=device)
-        _scratches[key] = buf
-    return buf
+    return need
 
 
 def _check_inputs(latents: Tensor, weight: Tensor) -> Tuple[int, int, int, int]:
@@ -73,7 +67,7 @@ def code_indices(latents: Tensor, weight: Tensor, mode: int = L.VQ_AUTO, debug_s
     E = weight.detach().contiguous()
     idx = torch.empty(B * HW, dtype=torch.int64, device=z.device)
     stream = L.stream_of(z)
-    ws = _workspace(z.device, B * HW, K, D, stream)
+    ws = _buffer("vq", z.device, stream, _workspace_bytes(B * HW, K, D))
     with torch.cuda.device(z.device):
         L.check(L.lib().movae_vq_argmin_f32(L.ptr(z), B, D, HW, L.ptr(E), K, L.ptr(idx), int(mode), L.ptr(debug_scores),
                                             L.ptr(ws), ws.numel(), stream), "vq_argmin_f32")
@@ -82,9 +76,9 @@ def code_indices(latents: Tensor, weight: Tensor, mode: int = L.VQ_AUTO, debug_s
 
 def rechecked_rows(device: torch.device) -> int:
     """Rows the last tensor-path search on the current stream re-evaluated exactly (synchronises)."""
-    key = (torch.device(device).index if torch.device(device).index is not None else torch.cuda.current_device(),
+    key = ("vq", torch.device(device).index if torch.device(device).index is not None else torch.cuda.current_device(),
            torch.cuda.current_stream(device).cuda_stream)
-    ws = _workspaces.get(key)
+    ws = _buffers.get(key)
     return 0 if ws is None else int(ws[:4].view(torch.int32).item())
 
 
@@ -94,10 +88,50 @@ def codebook_usage_count(encoding_inds: Tensor, K: int) -> Tensor:
     idx = encoding_inds.detach().reshape(-1).to(torch.int64).contiguous()
     out = torch.zeros(1, dtype=torch.int32, device=idx.device)
     stream = L.stream_of(idx)
-    ws = _workspace(idx.device, 0, K, 1, stream)
+    ws = _buffer("vq", idx.device, stream, _workspace_bytes(0, K, 1))
     with torch.cuda.device(idx.device):
         L.check(L.lib().movae_vq_usage(L.ptr(idx), idx.numel(), K, L.ptr(out), L.ptr(ws), ws.numel(), stream), "vq_usage")
     return out
+
+
+def _forward(latents: Tensor, E: Tensor, mode: int) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """K4 + K5 with the contiguous codebook E, on the current stream: (z, idx, quantized, losses [commitment, embedding],
+    usage)."""
+    B, D, HW, K = _check_inputs(latents, E)
+    z = latents.detach().contiguous()
+    N = B * HW
+    if N == 0:
+        raise RuntimeError("movae_b200: empty latents")
+    idx = torch.empty(N, dtype=torch.int64, device=z.device)
+    quantized = torch.empty_like(z)
+    losses = torch.empty(2, dtype=torch.float32, device=z.device)
+    usage = torch.empty(1, dtype=torch.int32, device=z.device)
+    stream = L.stream_of(z)
+    ws = _buffer("vq", z.device, stream, _workspace_bytes(N, K, D))
+    with torch.cuda.device(z.device):
+        L.check(L.lib().movae_vq_forward_f32(L.ptr(z), B, D, HW, L.ptr(E), K, L.ptr(idx), L.ptr(quantized), L.ptr(losses),
+                                             L.ptr(usage), int(mode), L.ptr(ws), ws.numel(), stream), "vq_forward_f32")
+    return z, idx, quantized, losses, usage
+
+
+def _backward(z: Tensor, E: Tensor, idx: Tensor, g_q: Optional[Tensor], g_commit: Optional[Tensor],
+              g_embed: Optional[Tensor], want_dz: bool) -> Tuple[Optional[Tensor], Optional[Tensor]]:
+    """K6 on the current stream: dz when `want_dz`, dE when `g_embed` is given (None: no codebook gradient)."""
+    B, D, H, W = z.shape
+    K = E.shape[0]
+    dz = torch.empty_like(z) if want_dz else None
+    dE = torch.zeros_like(E) if g_embed is not None else None
+    if dz is None and dE is None:
+        return None, None
+    f32 = lambda t: None if t is None else t.detach().to(torch.float32).contiguous()  # noqa: E731
+    g_q, g_commit, g_embed = f32(g_q), f32(g_commit), f32(g_embed)
+    stream = L.stream_of(z)
+    need = L.lib().movae_vq_backward_workspace_bytes(B * H * W, K, D) if dE is not None else 0
+    scratch = _buffer("k6", z.device, stream, need, zero=False) if need else None
+    with torch.cuda.device(z.device):
+        L.check(L.lib().movae_vq_backward_f32(L.ptr(g_q), L.ptr(g_commit), L.ptr(g_embed), L.ptr(z), B, D, H * W, L.ptr(E), K,
+                                              L.ptr(idx), L.ptr(dz), L.ptr(dE), L.ptr(scratch), need, stream), "vq_backward_f32")
+    return dz, dE
 
 
 class _Quantize(torch.autograd.Function):
@@ -107,21 +141,8 @@ class _Quantize(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, latents: Tensor, weight: Tensor, mode: int):
-        B, D, HW, K = _check_inputs(latents, weight)
-        z = latents.detach().contiguous()
         E = weight.detach().contiguous()
-        N = B * HW
-        if N == 0:
-            raise RuntimeError("movae_b200: empty latents")
-        idx = torch.empty(N, dtype=torch.int64, device=z.device)
-        quantized = torch.empty_like(z)
-        losses = torch.empty(2, dtype=torch.float32, device=z.device)
-        usage = torch.empty(1, dtype=torch.int32, device=z.device)
-        stream = L.stream_of(z)
-        ws = _workspace(z.device, N, K, D, stream)
-        with torch.cuda.device(z.device):
-            L.check(L.lib().movae_vq_forward_f32(L.ptr(z), B, D, HW, L.ptr(E), K, L.ptr(idx), L.ptr(quantized), L.ptr(losses),
-                                                 L.ptr(usage), int(mode), L.ptr(ws), ws.numel(), stream), "vq_forward_f32")
+        z, idx, quantized, losses, usage = _forward(latents, E, mode)
         ctx.save_for_backward(z, E, idx)
         ctx.set_materialize_grads(False)
         ctx.mark_non_differentiable(idx, usage)
@@ -130,27 +151,10 @@ class _Quantize(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_q, g_commit, g_embed, _g_idx, _g_usage):
         z, E, idx = ctx.saved_tensors
-        B, D, H, W = z.shape
-        K = E.shape[0]
-        need_z, need_E = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
-        dz = dE = None
-        if need_z and not (g_q is None and g_commit is None):
-            dz = torch.empty_like(z)      # else None: nothing reaches the latents (embedding_loss alone, vq_vae.py:52), and
-                                          # autograd reports the latents as unused instead of back-propagating zeros
-        run_E = need_E and g_embed is not None          # only embedding_loss reaches the codebook (vq_vae.py:51-55)
-        if run_E:
-            dE = torch.zeros_like(E)
-        if dz is not None or run_E:
-            f32 = lambda t: None if t is None else t.detach().to(torch.float32).contiguous()  # noqa: E731
-            g_q, g_commit, g_embed = f32(g_q), f32(g_commit), f32(g_embed)
-            scratch = None
-            need = L.lib().movae_vq_backward_workspace_bytes(B * H * W, K, D) if run_E else 0
-            if need:
-                scratch = _scratch(z.device, need, L.stream_of(z))
-            with torch.cuda.device(z.device):
-                L.check(L.lib().movae_vq_backward_f32(L.ptr(g_q), L.ptr(g_commit), L.ptr(g_embed), L.ptr(z), B, D, H * W, L.ptr(E),
-                                                      K, L.ptr(idx), L.ptr(dz), L.ptr(dE) if run_E else 0,
-                                                      L.ptr(scratch), need, L.stream_of(z)), "vq_backward_f32")
+        # no dz when nothing reaches the latents (embedding_loss alone, vq_vae.py:52): autograd then reports the latents
+        # as unused instead of back-propagating zeros.  Only embedding_loss reaches the codebook (vq_vae.py:51-55).
+        want_dz = ctx.needs_input_grad[0] and not (g_q is None and g_commit is None)
+        dz, dE = _backward(z, E, idx, g_q, g_commit, g_embed if ctx.needs_input_grad[1] else None, want_dz)
         return dz, dE, None
 
 
@@ -168,12 +172,14 @@ class VectorQuantizer(nn.Module):
         self.last_usage_count: Optional[Tensor] = None   # int32 device scalar written by K5's bitmap
 
     def forward(self, latents: Tensor):
-        quantized, commitment_loss, embedding_loss, encoding_inds, usage = _Quantize.apply(
-            latents, self.embedding.weight, self.search_mode)
+        quantized, commitment_loss, embedding_loss, encoding_inds, usage = self._quantize(latents)
         self.last_usage_count = usage
         if getattr(self, "_summary_mode", False):
             return quantized
         return quantized, commitment_loss, embedding_loss, encoding_inds
+
+    def _quantize(self, latents: Tensor):
+        return _Quantize.apply(latents, self.embedding.weight, self.search_mode)
 
     def embed_code(self, code: Tensor) -> Tensor:
         return self.embedding(code)
@@ -208,24 +214,10 @@ class _QuantizeEMA(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, latents: Tensor, vq: "VectorQuantizerEMA", update: bool):
-        weight = vq.embedding.weight
-        B, D, HW, K = _check_inputs(latents, weight)
-        z = latents.detach().contiguous()
-        E = weight.detach()
+        E = vq.embedding.weight.detach()
         if not E.is_contiguous():
             raise RuntimeError("movae_b200: VectorQuantizerEMA updates embedding.weight in place and needs it contiguous")
-        N = B * HW
-        if N == 0:
-            raise RuntimeError("movae_b200: empty latents")
-        idx = torch.empty(N, dtype=torch.int64, device=z.device)
-        quantized = torch.empty_like(z)
-        losses = torch.empty(2, dtype=torch.float32, device=z.device)
-        usage = torch.empty(1, dtype=torch.int32, device=z.device)
-        stream = L.stream_of(z)
-        ws = _workspace(z.device, N, K, D, stream)
-        with torch.cuda.device(z.device):
-            L.check(L.lib().movae_vq_forward_f32(L.ptr(z), B, D, HW, L.ptr(E), K, L.ptr(idx), L.ptr(quantized), L.ptr(losses),
-                                                 L.ptr(usage), int(vq.search_mode), L.ptr(ws), ws.numel(), stream), "vq_forward_f32")
+        z, idx, quantized, losses, usage = _forward(latents, E, vq.search_mode)
         if update:
             vq._update(z, idx)
             E = vq._pre_update
@@ -239,26 +231,8 @@ class _QuantizeEMA(torch.autograd.Function):
         z, E, idx = ctx.saved_tensors
         if not ctx.needs_input_grad[0] or (g_q is None and g_commit is None):
             return None, None, None
-        B, D, H, W = z.shape
-        dz = torch.empty_like(z)
-        f32 = lambda t: None if t is None else t.detach().to(torch.float32).contiguous()  # noqa: E731
-        g_q, g_commit = f32(g_q), f32(g_commit)
-        with torch.cuda.device(z.device):
-            L.check(L.lib().movae_vq_backward_f32(L.ptr(g_q), L.ptr(g_commit), 0, L.ptr(z), B, D, H * W, L.ptr(E), E.shape[0],
-                                                  L.ptr(idx), L.ptr(dz), 0, 0, 0, L.stream_of(z)), "vq_backward_f32")
+        dz, _ = _backward(z, E, idx, g_q, g_commit, None, True)
         return dz, None, None
-
-
-def _ema_workspace(device: torch.device, n_rows: int, K: int, D: int, stream: int) -> Tensor:
-    """Zero-initialised EMA workspace (ticket, stats, K6b partials), one per (device, stream), grown with the batch.  It
-    lives in the same cache as the quantizer workspaces, so GraphedStep keeps it alive with them."""
-    need = L.lib().movae_vq_ema_workspace_bytes(n_rows, K, D)
-    key = ("ema", device.index, stream)
-    ws = _workspaces.get(key)
-    if ws is None or ws.numel() < need:
-        ws = torch.zeros(need, dtype=torch.uint8, device=device)
-        _workspaces[key] = ws
-    return ws
 
 
 class VectorQuantizerEMA(VectorQuantizer):
@@ -312,12 +286,8 @@ class VectorQuantizerEMA(VectorQuantizer):
         self.stats_reducer: Optional[Callable[[Tensor], None]] = None
         self._stats: Optional[Tensor] = None
 
-    def forward(self, latents: Tensor):
-        quantized, commitment_loss, embedding_loss, encoding_inds, usage = _QuantizeEMA.apply(latents, self, self.training)
-        self.last_usage_count = usage
-        if getattr(self, "_summary_mode", False):
-            return quantized
-        return quantized, commitment_loss, embedding_loss, encoding_inds
+    def _quantize(self, latents: Tensor):
+        return _QuantizeEMA.apply(latents, self, self.training)
 
     def _update(self, z: Tensor, idx: Tensor) -> None:
         """The EMA update from the batch `z` [B, D, H, W] and its indices, on the current stream, no host synchronisation."""
@@ -328,8 +298,8 @@ class VectorQuantizerEMA(VectorQuantizer):
         B, D, H, W = z.shape
         K = self.K
         stream = L.stream_of(z)
-        ws = _ema_workspace(z.device, B * H * W, K, D, stream)
         lib = L.lib()
+        ws = _buffer("ema", z.device, stream, lib.movae_vq_ema_workspace_bytes(B * H * W, K, D))
         with torch.cuda.device(z.device):
             if self.stats_reducer is None:
                 L.check(lib.movae_vq_ema_update_f32(L.ptr(z), B, D, H * W, L.ptr(idx), K, self.decay, self.epsilon, L.ptr(E),
