@@ -18,7 +18,11 @@
 // R rows x 1 FMA and four codes per lane run as independent chains (the one-row version was
 // shared-memory-bandwidth bound: 1300 wavefronts per row).  Two-stage evaluation: a float32 FMA pass
 // over all K codes selects the candidates whose score is within a safe bound of the row minimum, only
-// those are re-evaluated with float64 sums.
+// those are re-evaluated with float64 sums.  Inf / NaN latents or codebook entries make the bound non-finite and every
+// code a candidate; as in torch.argmin the first NaN distance wins.
+//
+// Limits at D = 64: the staged variant (R = 4) up to K = 558, the unstaged one (R = 1, codebook read from global memory)
+// up to K = 6,200; larger codebooks are MOVAE_ERR_UNSUPPORTED.
 #include <math.h>
 
 #include "common.cuh"
@@ -97,8 +101,13 @@ vq_argmin_exact_kernel(const float* __restrict__ z, int64_t N, int D, int64_t HW
     }
     __syncthreads();
     float emax2 = 0.f;
-    for (int j = lane; j < K; j += 32) emax2 = fmaxf(emax2, e2s[j]);
+    bool finite_e = true;
+    for (int j = lane; j < K; j += 32) {
+        emax2 = fmaxf(emax2, e2s[j]);
+        finite_e = finite_e && e2s[j] <= 3.4028235e38f;
+    }
     emax2 = -warp_min_f(-emax2);
+    if (!__all_sync(0xffffffffu, finite_e)) emax2 = __uint_as_float(0x7fc00000u);   // NaN bound: every row evaluates every code
     const float emax = sqrtf(emax2);
 
     for (int64_t g = (int64_t)blockIdx.x * kExWarps + warp; g < n_groups; g += stride) {
@@ -210,11 +219,14 @@ vq_argmin_exact_kernel(const float* __restrict__ z, int64_t N, int D, int64_t HW
             // formula's own quantum, 8 ulp of |z|^2 + |e|^2) of the minimum can be the float32-rounded argmin
             const float bound = 2.f * (float)(D + 2) * 5.9604645e-08f * (2.f * znorm * emax + emax2) +
                                 8.f * 1.1920929e-07f * (z2f[r] + emax2);
+            const float lim = b32 + bound;
+            // inf / NaN latents or codebook rows: the limit bounds nothing and every code is evaluated
+            const bool all = !(fabsf(lim) <= 3.4028235e38f);
             float bestd = __uint_as_float(0x7f800000u);
             int bestj = 0x7fffffff;
             for (int jb = 0; jb < K; jb += 32) {
                 const int j = jb + lane;
-                unsigned cand = __ballot_sync(0xffffffffu, j < K && sc[r * K + j] <= b32 + bound);
+                unsigned cand = __ballot_sync(0xffffffffu, j < K && (all || sc[r * K + j] <= lim));
                 while (cand) {                                  // the whole warp evaluates one candidate: lanes over d
                     const int jc = jb + __ffs(cand) - 1;
                     cand &= cand - 1;
@@ -227,10 +239,12 @@ vq_argmin_exact_kernel(const float* __restrict__ z, int64_t N, int D, int64_t HW
                     dd = warp_sum(dd);
                     ee = warp_sum(ee);
                     const float dist = __fsub_rn(__fadd_rn(z2f[r], (float)ee), __fmul_rn(2.f, (float)dd));
-                    if (dist < bestd) { bestd = dist; bestj = jc; }   // candidates visited in ascending j: first minimum kept
+                    // candidates visited in ascending j: first minimum kept, and as in torch.argmin the first NaN beats
+                    // everything
+                    if (dist < bestd || (dist != dist && bestd == bestd)) { bestd = dist; bestj = jc; }
                 }
             }
-            // every distance inf / NaN (non-finite latents): torch.argmin of such a row is its first element
+            // every distance inf: torch.argmin of such a row is its first element
             if (lane == 0) idx_out[rows[r]] = (long long)(bestj == 0x7fffffff ? 0 : bestj);
         }
         __syncwarp();

@@ -31,8 +31,11 @@
 // error 2 * 2^-15 max|z| max|e| <= M 2^-16, plus 4 rounding quanta of 8 u) goes onto a shared-memory ring
 // and is re-evaluated exactly (reference formula, float32 roundings) INSIDE this kernel by two re-check
 // warps (round 1 ran a second kernel over a global worklist: 16 us of fixed cost at N = 8,192, 92 us at
-// N = 4.2 M).  Every other row provably has the same argmin as exact
-// arithmetic.
+// N = 4.2 M).  M also exceeds 2 C + (max|z|^2 + max|e|^2) / 32 over the tile, so every other row provably has the
+// same argmin as the reference formula with its float32 roundings (first minimal index).  Non-finite inputs: a
+// codebook with an inf / NaN entry sends every row to the full re-check; inf / NaN latents make their tile's keys
+// inf / NaN, which the epilogue's !(a - b > thr) tests count as close, so those rows are re-checked too.  The re-check
+// follows torch.argmin: the first NaN distance wins.
 //
 // Roofline: tensor pipe.  Algorithmic work 2*K*D = 65,536 flop per code vector; executed 15/4 of that
 // (three bf16 products + three key steps).  HBM traffic 4*D = 256 B read + 8 B written per code vector.
@@ -102,7 +105,8 @@ __device__ __forceinline__ int ld_volatile_i32(const int* p) { return *reinterpr
 // all 512 codes that reads the RESIDENT operand image: hi(-2E) alone (bf16: relative error 2^-9 per element, so the
 // candidate bound is 2 * 2^-8 |z| max|e| on top of the float32 pass's own error -- a superset of what the exact kernel
 // would select; typically 2-3 codes) plus |e|^2 from the side table.  Each candidate is then evaluated by the lane that
-// owns it from the float32 codebook in global memory (L2-resident).
+// owns it from the float32 codebook in global memory (L2-resident).  When the bound is not finite (inf / NaN latents or
+// codebook) every code is a candidate.
 __device__ __noinline__ void recheck_row_in_kernel(int4 ent, const float* __restrict__ z, int64_t HW, const float* __restrict__ E,
                                                     const uint8_t* smem, float* zs, float emax, float emax2,
                                                     long long* __restrict__ idx_out, unsigned int* __restrict__ count, int lane) {
@@ -116,10 +120,9 @@ __device__ __noinline__ void recheck_row_in_kernel(int4 ent, const float* __rest
     const float z2f = (float)warp_sum((double)za * (double)za + (double)zb * (double)zb);
     __syncwarp();
     if (lane == 0) atomicAdd(count, 1u);
-    if (!(z2f <= 3.4028234e38f)) {                 // |z|^2 overflows or is NaN: every distance is inf / NaN -> code 0, like the exact kernel
-        if (lane == 0) idx_out[n] = 0;
-        return;
-    }
+    // torch.argmin's order: a NaN distance is smaller than everything (the first NaN wins), inf never wins over a finite
+    // distance, and a row whose distances are all inf gets code 0
+    auto key_of = [](float dist, int j) { return dist != dist ? (unsigned long long)j : pack_dist_index(dist, j); };
     if (ent.y > 0) {
         // ---- the epilogue knows every candidate (<= 4 codes, one per tracker): evaluate just those, lanes over channels ----
         const int codes[4] = {ent.z & 0xFFFF, (ent.z >> 16) & 0xFFFF, ent.w & 0xFFFF, (ent.w >> 16) & 0xFFFF};
@@ -137,8 +140,8 @@ __device__ __noinline__ void recheck_row_in_kernel(int4 ent, const float* __rest
                 const double dd = warp_sum(fma((double)e0[i], (double)za, (double)e1[i] * (double)zb));
                 const double ee = warp_sum(fma((double)e0[i], (double)e0[i], (double)e1[i] * (double)e1[i]));
                 const float dist = __fsub_rn(__fadd_rn(z2f, (float)ee), __fmul_rn(2.f, (float)dd));
-                if (dist < __uint_as_float(0x7f800000u)) {
-                    const unsigned long long key = pack_dist_index(dist, codes[i]);
+                if (!(dist >= __uint_as_float(0x7f800000u))) {
+                    const unsigned long long key = key_of(dist, codes[i]);
                     bestk = key < bestk ? key : bestk;
                 }
             }
@@ -180,11 +183,14 @@ __device__ __noinline__ void recheck_row_in_kernel(int4 ent, const float* __rest
     const float znorm = sqrtf(z2f);
     const float bound = 2.02f * 0.00390625f * znorm * emax +
                         2.f * (float)(kTcD + 2) * 5.9604645e-08f * (2.f * znorm * emax + emax2) + 8.f * 1.1920929e-07f * (z2f + emax2);
+    // a non-finite limit (inf / NaN latents or codebook rows) bounds nothing: every code is evaluated
+    const float lim = fabsf(mn + bound) <= 3.4028235e38f ? mn + bound : __uint_as_float(0x7f800000u);
     // ---- pass 2: this lane's candidates with float64 sums and the reference's float32 formula ----
     unsigned long long best = ~0ull;
+    int nan_j = kTcK;                                      // first code with a NaN distance (kTcK: none)
 #pragma unroll 1
     for (int c = 0; c < 16; ++c) {
-        if (acc[c] <= mn + bound) {
+        if (!(acc[c] > lim)) {
             const int j = lane + 32 * c;
             const float* ep = E + (size_t)j * kTcD;
             double dd = 0.0, ee = 0.0;
@@ -201,18 +207,21 @@ __device__ __noinline__ void recheck_row_in_kernel(int4 ent, const float* __rest
                 dd = fma((double)e.w, (double)q.w, dd); ee = fma((double)e.w, (double)e.w, ee);
             }
             const float dist = __fsub_rn(__fadd_rn(z2f, (float)ee), __fmul_rn(2.f, (float)dd));
-            if (dist < __uint_as_float(0x7f800000u)) {     // inf / NaN distances never win (index 0 if nothing does)
+            if (dist < __uint_as_float(0x7f800000u)) {     // inf never wins (index 0 if every distance is inf)
                 const unsigned long long key = pack_dist_index(dist, j);
                 best = key < best ? key : best;            // smallest distance, then smallest index
             }
+            if (dist != dist) nan_j = min(nan_j, j);
         }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         const unsigned long long other = __shfl_xor_sync(0xffffffffu, best, o);
         best = other < best ? other : best;
+        nan_j = min(nan_j, __shfl_xor_sync(0xffffffffu, nan_j, o));
     }
-    if (lane == 0) idx_out[n] = best == ~0ull ? 0ll : (long long)(unsigned int)(best & 0xffffffffull);
+    if (lane == 0)
+        idx_out[n] = nan_j < kTcK ? (long long)nan_j : best == ~0ull ? 0ll : (long long)(unsigned int)(best & 0xffffffffull);
 }
 
 // One attempt to take a row off the re-check ring and re-evaluate it (warp-collective).  Returns false when the ring was
@@ -403,9 +412,17 @@ vq_argmin_tc_kernel(const float* __restrict__ z, int64_t N, int64_t HW, const fl
                 const float z2max = fmaxf(fmaxf(bars->pmax[s][0], bars->pmax[s][1]), fmaxf(bars->pmax[s][2], bars->pmax[s][3]));
                 // C >= 2 |z||e| (1 + 5e-4) rounded UP to bf16; score + C in (0, Rg) with Rg = 2 C + max|e|^2
                 const float Craw = 2.001f * sqrtf(z2max * 1.00001f) * emax + 1e-30f;
-                const uint32_t Cb = (__float_as_uint(Craw) + 0xFFFFu) >> 16;
+                uint32_t Cb = (__float_as_uint(Craw) + 0xFFFFu) >> 16;
                 const float C = __uint_as_float(Cb << 16);
-                const float Rg = fmaxf(2.f * C + emax2, 1e-30f) * 1.001f;
+                // M 2^-16 >= 2C 2^-16 (the tensor-path error) + 2^-21 (|z|^2 + |e|^2), what the reference formula's float32
+                // roundings (<= 2^-22 (|z|^2 + |e|^2) per distance) can reverse, so a row decided on the tensor path gets
+                // the formula's first minimum even when |z| >> |e| makes its distances round together.  max|e|^2, which the
+                // key range needs anyway, covers that term unless |z|^2 > 31 max|e|^2.
+                const float Rg = fmaxf(2.f * C + fmaxf(emax2, 0.03125f * (z2max + emax2)), 1e-30f) * 1.001f;
+                // an inf / NaN codebook entry (atomicMax on the bits carries it into emax2) or |z|^2 overflowing float32
+                // leaves no key scale: C = NaN makes every key of the tile NaN, and the epilogue sends every row to the
+                // full re-check (NaN keys count as close), where the first NaN distance wins as in torch.argmin
+                if (!(emax2 <= 3.4028235e38f) || !(Rg <= 3.4028235e38f)) Cb = 0x7FC0u;
                 uint32_t mexp = (__float_as_uint(Rg) >> 23) + 1u;            // M = 2^m > Rg
                 mexp = mexp < 40u ? 40u : mexp;                              // keep u = M 2^-23 a normal number
                 const uint32_t M_hi = mexp << 7;                             // bf16 bits of M

@@ -200,8 +200,9 @@ def test_large_search_staged_recheck_matches_exact_mode(mv, codebook):
 @pytest.mark.parametrize("shape", [(4, 8, 8), (40, 64, 64)], ids=["direct_recheck", "N163840"])
 def test_non_finite_and_huge_latents_stay_in_range(mv, ov, shape):
     """Diverged training (the reference only warns, main.py:163-164): rows with inf / NaN / overflowing latents must not crash
-    or produce out-of-range indices; rows whose float32 distances all overflow to inf select code 0 like torch.argmin; every
-    finite row keeps its exact index."""
+    or produce out-of-range indices; every non-finite row gets torch.argmin's index (the first NaN distance, or code 0 when
+    every distance overflows to inf -- decided by where the inf / NaN terms fall, not by rounding); every finite row keeps
+    its exact index."""
     B, H, W = shape
     z, E = make_inputs(B, 64, H, W, 512, "trained", seed=99)
     z[0, :, 0, 0] = float("inf")
@@ -217,6 +218,7 @@ def test_non_finite_and_huge_latents_stay_in_range(mv, ov, shape):
     HW = H * W
     assert int(idx[1 * HW + 2 * W + 3]) == 0 == int(ref[1 * HW + 2 * W + 3])
     finite = torch.isfinite(z).all(dim=1).reshape(-1) & (z.abs().amax(dim=1).reshape(-1) < 1e18)
+    assert int((~finite).sum()) == 4 and torch.equal(idx[~finite], ref[~finite])
     ties = ov.tie_rows(torch.nan_to_num(z, nan=0.0, posinf=0.0, neginf=0.0).clamp(-10, 10), E)
     assert not bool(((idx != ref) & finite & ~ties).any())
 
