@@ -24,7 +24,7 @@ autograd (not ours); what changes is everything after them:
 """
 from __future__ import annotations
 
-from typing import Iterable, List, Optional, Sequence
+from typing import Callable, Iterable, Iterator, List, Optional, Sequence, Tuple
 
 import torch
 from torch import Tensor
@@ -33,12 +33,6 @@ from .aggregation import Aggregator
 from .optim import flat_plan
 
 _J_CACHE: dict = {}
-
-# Jacobian rows by k sequential backward passes (default) or by ONE batched (vmapped) pass over the live objectives like
-# torchjd's default (parallel_chunk_size=None).  Measured on B200 (tools/step_probe.py, BASELINE model configs, step under a
-# CUDA graph): sequential 2.57 / 14.98 / 21.92 ms vs batched 2.64 / 15.97 / 23.11 ms per step (VQ-VAE / GG-VQ-VAE / VQ-VAE2)
-# -- the vmapped convolution-backward costs more than the launches it saves.
-BATCHED_JACOBIAN = False
 
 
 def _leaves_of(roots: Sequence[Tensor], stop_at: Sequence[Tensor] = ()) -> List[Tensor]:
@@ -105,94 +99,44 @@ def _fill_row(J: Tensor, i: int, params: Sequence[Tensor], grads: Sequence[Optio
         torch._foreach_copy_(dst, src)
 
 
-def _fill_rows_batched(J: Tensor, rows: Sequence[int], params: Sequence[Tensor], grads: Sequence[Optional[Tensor]],
-                       offsets: Sequence[int]) -> None:
-    """grads[p]: [len(rows), *p.shape] (or None) -> columns off..off+numel of rows `rows` of J, one strided copy each."""
-    r = len(rows)
-    whole = list(rows) == list(range(J.shape[0]))
-    Jr = J if whole else None
-    dst, src = [], []
-    for p, g, off in zip(params, grads, offsets):
-        n = p.numel()
-        if whole:
-            view = Jr[:, off:off + n]
-        elif list(rows) == list(range(rows[0], rows[0] + r)):
-            view = J[rows[0]:rows[0] + r, off:off + n]
-        else:
-            view = None
-        if view is not None:
-            if g is None:
-                view.zero_()
-            else:
-                dst.append(view)
-                src.append(g.reshape(r, n))
-        else:                                             # non-consecutive live rows: one copy per row
-            for a, i in enumerate(rows):
-                if g is None:
-                    J[i, off:off + n].zero_()
-                else:
-                    dst.append(J[i, off:off + n])
-                    src.append(g[a].reshape(n))
-    if dst:
-        torch._foreach_copy_(dst, src)
-
-
-def _jacobian_rows(J: Tensor, outputs: Sequence[Tensor], params: Sequence[Tensor], grad_outputs_per_row: Sequence[Optional[Sequence[Tensor]]],
-                   retain_graph: bool, offsets: Optional[Sequence[int]] = None, dp=None) -> None:
-    """Fills J[i] = d(sum_j <outputs[j], grad_outputs_per_row[i][j]>) / d params for every row i; a row whose
-    entry is None is identically zero (no backward pass).  With a data-parallel plan (`dp`) every finished row is
-    handed to it at once, so its reduce-scatter overlaps the backward pass of the next row."""
-    offsets = _dense_offsets(params) if offsets is None else offsets
-    Jp = None
-    if dp is not None:
-        kk, P = J.shape
-        padded = dp.padded_columns(P)
-        Jp = J.as_strided((kk, padded), (J.stride(0) if kk > 1 else padded, 1))
-        dp.begin_rows(kk, P, J.dtype, J.device)
-    live = [i for i, g in enumerate(grad_outputs_per_row) if g is not None]
+def _row_gradients(outputs: Sequence, params: Sequence[Tensor], grad_outputs_per_row: Sequence[Optional[Sequence[Tensor]]],
+                   retain_graph: bool) -> Iterator[Tuple[int, Optional[Sequence[Optional[Tensor]]]]]:
+    """Yields (i, grads) in row order: the tuple autograd returns for d(sum_j <outputs[j], grad_outputs_per_row[i][j]>) / d params
+    (entries may be None), or None for an identically zero row (no backward pass).  `outputs[i]` is row i's own list when
+    every row differentiates its own scalar (`backward`).  Row i's pass runs when the consumer asks for it, so whatever
+    the consumer does with row i-1 is enqueued before it."""
+    # One backward pass per row.  One vmapped pass over all rows (torchjd's default) measured slower on every BASELINE model
+    # config, per step under a CUDA graph on one B200 (power limit not recorded): 2.64 / 15.97 / 23.11 ms against
+    # 2.57 / 14.98 / 21.92 ms for VQ-VAE / GG-VQ-VAE / VQ-VAE2 -- the vmapped convolution backward costs more than the
+    # launches it saves.
+    per_row = isinstance(outputs[0], (list, tuple))
+    last = max((i for i, g in enumerate(grad_outputs_per_row) if g is not None), default=-1)
     for i, g in enumerate(grad_outputs_per_row):
         if g is None:
+            yield i, None
+        else:
+            yield i, torch.autograd.grad(outputs[i] if per_row else outputs, params, grad_outputs=list(g),
+                                         retain_graph=retain_graph or i < last, allow_unused=True)
+
+
+def _fill_jacobian(J: Tensor, rows, params: Sequence[Tensor], offsets: Sequence[int], dp=None) -> None:
+    """J[i] from row i's gradients (an identically zero row is one memset).  With a data-parallel plan (`dp`) every
+    finished row is handed to it before the next row's backward pass runs, so its reduce-scatter overlaps that pass."""
+    if dp is not None:
+        k, P = J.shape
+        padded = dp.padded_columns(P)
+        Jp = J.as_strided((k, padded), (J.stride(0) if k > 1 else padded, 1))
+        dp.begin_rows(k, P, J.dtype, J.device)
+    for i, grads in rows:
+        if grads is None:
             J[i].zero_()
-            if dp is not None:
-                dp.row_zero(i)
-    k = len(live)
-    if k == 0:
-        return
-    if BATCHED_JACOBIAN and k > 1 and not isinstance(outputs[0], (list, tuple)):
-        try:
-            stacked = [torch.stack([grad_outputs_per_row[i][j] for i in live]) for j in range(len(outputs))]
-            grads = torch.autograd.grad(outputs, params, grad_outputs=stacked, retain_graph=True, allow_unused=True,
-                                        is_grads_batched=True)
-            _fill_rows_batched(J, live, params, grads, offsets)
-            if dp is not None:
-                for i in live:
-                    dp.row_ready(i, Jp[i])
-            return            # the graph is released with the last reference; torchjd keeps the same contract
-        except RuntimeError as e:                         # no batching rule somewhere in the graph
-            if "cuda" in str(e).lower() and "vmap" not in str(e).lower() and "batching" not in str(e).lower():
-                raise
-    per_row = isinstance(outputs[0], (list, tuple))
-    for a, i in enumerate(live):
-        keep = retain_graph or a < k - 1
-        grads = torch.autograd.grad(outputs[i] if per_row else outputs, params, grad_outputs=list(grad_outputs_per_row[i]),
-                                    retain_graph=keep, allow_unused=True)
-        _fill_row(J, i, params, grads, offsets)
+        else:
+            _fill_row(J, i, params, grads, offsets)
         if dp is not None:
-            dp.row_ready(i, Jp[i])
-
-
-def _row_gradients(outputs: Sequence[Tensor], params: Sequence[Tensor], grad_outputs_per_row: Sequence[Optional[Sequence[Tensor]]],
-                   retain_graph: bool) -> List[Optional[Sequence[Optional[Tensor]]]]:
-    """Per row i: the tuple autograd returns for d(sum_j <outputs[j], grad_outputs_per_row[i][j]>) / d params (entries may be
-    None), or None for an identically zero row (no backward pass).  `outputs[j]` may be per-row (a list of lists) when
-    every row differentiates its own scalar (`backward`)."""
-    live = [i for i, g in enumerate(grad_outputs_per_row) if g is not None]
-    out: List[Optional[Sequence[Optional[Tensor]]]] = [None] * len(grad_outputs_per_row)
-    for a, i in enumerate(live):
-        keep = retain_graph or a < len(live) - 1
-        outs_i = outputs[i] if isinstance(outputs[0], (list, tuple)) else outputs
-        out[i] = torch.autograd.grad(outs_i, params, grad_outputs=list(grad_outputs_per_row[i]), retain_graph=keep, allow_unused=True)
-    return out
+            if grads is None:
+                dp.row_zero(i)
+            else:
+                dp.row_ready(i, Jp[i])
 
 
 _ZEROS: dict = {}
@@ -207,24 +151,16 @@ def _zero_row(device: torch.device, n: int) -> Tensor:
     return z
 
 
-def _segments_possible(params: Sequence[Tensor], aggregator) -> bool:
-    from . import _lib as L
-
-    return (not BATCHED_JACOBIAN and _dp_of(aggregator) is None and len(params) <= L.MAX_SEGMENTS
-            and hasattr(aggregator, "supports_segments") and aggregator.supports_segments())
-
-
-def _aggregate_segments_and_accumulate(row_grads, params: Sequence[Tensor], cols: Sequence[int], aggregator, plan) -> Tensor:
-    """The fused launch over the gradient tensors themselves; `.grad` semantics as _aggregate_and_accumulate."""
+def _segment_rows(rows, params: Sequence[Tensor]) -> List[List[Tensor]]:
+    """Every row as the list of gradient tensors the segmented launch reads in place; a missing gradient, and every entry
+    of an identically zero row, is the shared zero buffer."""
     from . import ops
 
-    dev = params[0].device
-    numels = [p.numel() for p in params]
-    zero = _zero_row(dev, max(numels))
-    rows = []
-    for gs in row_grads:
+    zero = _zero_row(params[0].device, max(p.numel() for p in params))
+    out = []
+    for _, gs in rows:
         if gs is None:
-            rows.append([zero] * len(params))
+            out.append([zero] * len(params))
             continue
         r = []
         for g in gs:
@@ -233,50 +169,44 @@ def _aggregate_segments_and_accumulate(row_grads, params: Sequence[Tensor], cols
             else:
                 g = g.detach()
                 r.append(g if ops.segment_ok(g) else g.to(torch.float32).contiguous().clone())     # rare: a strided / unaligned gradient
-        rows.append(r)
+        out.append(r)
+    return out
+
+
+def _segments_possible(params: Sequence[Tensor], aggregator) -> bool:
+    from . import _lib as L
+
+    return (_dp_of(aggregator) is None and len(params) <= L.MAX_SEGMENTS
+            and hasattr(aggregator, "supports_segments") and aggregator.supports_segments())
+
+
+def _write_back(params: Sequence[Tensor], cols: Sequence[int], P: int, plan, launch: Callable[[Tensor, bool], Tensor]) -> None:
+    """torchjd's Accumulate rule for the aggregated gradient: `launch(out, accumulate)` writes (or adds) it into `out`, with
+    params[j] at columns cols[j]..cols[j]+numel, and each `.grad` is assigned when None, added to otherwise.  When the
+    parameters are a run of a FlatParameters layout (`plan`; `cols` are then its columns) and every `.grad` is None, or
+    every `.grad` is already its view, `out` is the persistent flat gradient buffer the fused optimizer step (K7) reads;
+    otherwise it is a fresh buffer of P columns."""
     if plan is not None:
         owner, _, _, lo, hi = plan
         states = {owner.grad_state(p) for p in params}
         if states == {"none"}:
-            w = aggregator.aggregate_segments_into(rows, numels, cols, owner.flat_grad[lo:hi], accumulate=False)
+            launch(owner.flat_grad[lo:hi], False)
             for p in params:
                 p.grad = owner.grad_view(p)
-            return w
+            return
         if states == {"view"}:
-            return aggregator.aggregate_segments_into(rows, numels, cols, owner.flat_grad[lo:hi], accumulate=True)
-    # plain parameters (or mixed .grad states): a fresh flat buffer with every tensor on a 16-byte boundary
-    offs, off = [], 0
-    for n in numels:
-        offs.append(off)
-        off += (n + 3) // 4 * 4
-    flat = torch.empty(max(off, 4), dtype=torch.float32, device=dev)
-    w = aggregator.aggregate_segments_into(rows, numels, offs, flat, accumulate=False)
+            launch(owner.flat_grad[lo:hi], True)
+            return
+    flat = torch.empty(P, dtype=torch.float32, device=params[0].device)
+    launch(flat, False)
     add_dst, add_src = [], []
-    for p, o, n in zip(params, offs, numels):
-        g = flat[o:o + n].view(p.shape)
+    for p, off in zip(params, cols):
+        g = flat[off:off + p.numel()].view(p.shape)
         if p.grad is None:
             p.grad = g
         else:
             add_dst.append(p.grad)
             add_src.append(g)
-    if add_dst:
-        torch._foreach_add_(add_dst, add_src)
-    return w
-
-
-def _accumulate_flat(params: Sequence[Tensor], flat: Tensor) -> None:
-    """torchjd Accumulate: `p.grad = g` if None else `p.grad += g`; g are views of the flat buffer."""
-    off = 0
-    add_dst, add_src = [], []
-    for p in params:
-        n = p.numel()
-        g = flat[off:off + n].view(p.shape)
-        if p.grad is None:
-            p.grad = g
-        else:
-            add_dst.append(p.grad)
-            add_src.append(g)
-        off += n
     if add_dst:
         torch._foreach_add_(add_dst, add_src)
 
@@ -298,36 +228,6 @@ def _run_aggregation(J: Tensor, aggregator: Aggregator, out: Tensor, accumulate:
     return dp.aggregate_rows_into(J.shape[1], out, accumulate)     # the rows were handed over while they were built
 
 
-def _aggregate_and_accumulate(J: Tensor, params: Sequence[Tensor], aggregator: Aggregator, plan=None) -> Tensor:
-    if plan is not None:
-        # the parameters are a run of a FlatParameters layout and J's columns follow it: K3 writes (or adds)
-        # straight into the persistent flat gradient buffer the optimizer kernel reads
-        owner, _, _, lo, hi = plan
-        states = {owner.grad_state(p) for p in params}
-        if states == {"none"}:
-            w = _run_aggregation(J, aggregator, owner.flat_grad[lo:hi], False)
-            for p in params:
-                p.grad = owner.grad_view(p)
-            return w
-        if states == {"view"}:
-            return _run_aggregation(J, aggregator, owner.flat_grad[lo:hi], True)
-        cols = plan[2]
-        flat = torch.empty(J.shape[1], dtype=torch.float32, device=J.device)
-        w = _run_aggregation(J, aggregator, flat, False)
-        for p, off in zip(params, cols):
-            g = flat[off:off + p.numel()].view(p.shape)
-            if p.grad is None:
-                p.grad = g
-            else:
-                p.grad += g
-        return w
-    P = J.shape[1]
-    flat = torch.empty(P, dtype=torch.float32, device=J.device)
-    w = _run_aggregation(J, aggregator, flat, False)
-    _accumulate_flat(params, flat)
-    return w
-
-
 def _layout(params: Sequence[Tensor]):
     """(params in J's column order, column offsets, P, plan, cache key)."""
     plan = flat_plan(params)
@@ -338,10 +238,35 @@ def _layout(params: Sequence[Tensor]):
     return params, _dense_offsets(params), sum(p.numel() for p in params), None, ()
 
 
+def _aggregate_rows(outputs: Sequence, params: Sequence[Tensor], grad_outputs_per_row: Sequence[Optional[Sequence[Tensor]]],
+                    retain_graph: bool, aggregator) -> None:
+    """The rows of `_row_gradients` aggregated into the parameters' `.grad`: by the segmented launch over the gradient
+    tensors themselves when nothing needs a [k, P] matrix, else through the flat J."""
+    params, cols, P, plan, key = _layout(params)
+    if P == 0:
+        return
+    rows = _row_gradients(outputs, params, grad_outputs_per_row, retain_graph)
+    if _segments_possible(params, aggregator):
+        numels = [p.numel() for p in params]
+        seg = _segment_rows(rows, params)
+        if plan is None:                                  # every tensor on a 16-byte boundary, as a FlatParameters layout has it
+            cols, P = [], 0
+            for n in numels:
+                cols.append(P)
+                P += (n + 3) // 4 * 4
+        _write_back(params, cols, P, plan, lambda out, acc: aggregator.aggregate_segments_into(seg, numels, cols, out, accumulate=acc))
+        return
+    dp = _dp_of(aggregator)
+    J = _jacobian_buffer(len(grad_outputs_per_row), P, params[0].device, key, dp.padded_columns(P) if dp else 0)
+    _fill_jacobian(J, rows, params, cols, dp)
+    _write_back(params, cols, P, plan, lambda out, acc: _run_aggregation(J, aggregator, out, acc))
+
+
 def backward(tensors: Sequence[Tensor] | Tensor, aggregator: Aggregator, inputs: Optional[Iterable[Tensor]] = None,
              retain_graph: bool = False, parallel_chunk_size: Optional[int] = None) -> None:
     """Jacobian of `tensors` (k scalar losses) w.r.t. `inputs` (default: every leaf that requires
-    grad in their graph), aggregated into `.grad` (main.py:196)."""
+    grad in their graph), aggregated into `.grad` (main.py:196).  `parallel_chunk_size` is accepted for torchjd's
+    signature and ignored: the rows are always k sequential backward passes."""
     _check_aggregator(aggregator)
     losses = [tensors] if isinstance(tensors, Tensor) else list(tensors)
     if len(losses) == 0:
@@ -352,19 +277,11 @@ def backward(tensors: Sequence[Tensor] | Tensor, aggregator: Aggregator, inputs:
     params = list(inputs) if inputs is not None else _leaves_of(losses)
     if not params:
         return
-    k = len(losses)
-    params, cols, P, plan, key = _layout(params)
-    dp = _dp_of(aggregator)
     # every row differentiates ITS OWN loss: a stacked loss with one-hot cotangents would walk the union graph of all
     # objectives k times and push zero cotangents through the other objectives' private subgraphs (0 * inf = NaN)
     outputs = [[t.reshape(())] for t in losses]
     ones = [[torch.ones((), dtype=t.dtype, device=t.device)] for t in losses]
-    if _segments_possible(params, aggregator):
-        _aggregate_segments_and_accumulate(_row_gradients(outputs, params, ones, retain_graph), params, cols, aggregator, plan)
-        return
-    J = _jacobian_buffer(k, P, params[0].device, key, dp.padded_columns(P) if dp else 0)
-    _jacobian_rows(J, outputs, params, ones, retain_graph, cols, dp)
-    _aggregate_and_accumulate(J, params, aggregator, plan)
+    _aggregate_rows(outputs, params, ones, retain_graph, aggregator)
 
 
 def mtl_backward(losses: Sequence[Tensor], features: Sequence[Tensor] | Tensor, aggregator: Aggregator,
@@ -374,7 +291,7 @@ def mtl_backward(losses: Sequence[Tensor], features: Sequence[Tensor] | Tensor, 
     """Multi-task variant (main.py:188-194): task-specific parameters receive the plain SUM of
     their losses' gradients; the shared parameters (those the features depend on) receive the
     aggregation of the k rows  d loss_i / d shared  obtained by back-propagating each loss's
-    feature gradients through the shared part."""
+    feature gradients through the shared part.  `parallel_chunk_size` is accepted for torchjd's signature and ignored."""
     _check_aggregator(aggregator)
     losses = list(losses)
     feats = [features] if isinstance(features, Tensor) else list(features)
@@ -390,7 +307,6 @@ def mtl_backward(losses: Sequence[Tensor], features: Sequence[Tensor] | Tensor, 
         tasks = [list(tp) for tp in tasks_params]
         if len(tasks) != len(losses):
             raise ValueError("`tasks_params` must have one entry per loss")
-    k = len(losses)
 
     dp = _dp_of(aggregator)
     feat_grads: List[Optional[List[Tensor]]] = []
@@ -429,22 +345,5 @@ def mtl_backward(losses: Sequence[Tensor], features: Sequence[Tensor] | Tensor, 
     for owner, ps, gs in fresh_flat.values():
         owner.adopt(ps, gs)
         if dp is not None:
-            idx = sorted(p._movae_flat[1] for p in ps)
-            runs, start, prev = [], idx[0], idx[0]
-            for i in idx[1:] + [None]:
-                if i is None or i != prev + 1:
-                    runs.append(owner.flat_grad[owner.offsets[start]:owner.offsets[prev] + owner.padded_numel(prev)])
-                    start = i
-                prev = i if i is not None else prev
-            dp.average_(runs)
-    if not shared:
-        return
-    shared, cols, P, plan, key = _layout(shared)
-    if P == 0:
-        return
-    if _segments_possible(shared, aggregator):
-        _aggregate_segments_and_accumulate(_row_gradients(feats, shared, feat_grads, retain_graph), shared, cols, aggregator, plan)
-        return
-    J = _jacobian_buffer(k, P, shared[0].device, key, dp.padded_columns(P) if dp else 0)
-    _jacobian_rows(J, feats, shared, feat_grads, retain_graph, cols, dp)
-    _aggregate_and_accumulate(J, shared, aggregator, plan)
+            dp.average_([owner.flat_grad[lo:hi] for lo, hi in owner.runs(p._movae_flat[1] for p in ps)])
+    _aggregate_rows(feats, shared, feat_grads, retain_graph, aggregator)

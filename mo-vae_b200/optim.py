@@ -105,6 +105,18 @@ class FlatParameters:
         ordered = [self.params[i] for i in idx]
         return ordered, [self.offsets[i] - lo for i in idx], lo, hi
 
+    def runs(self, indices: Iterable[int]) -> List[Tuple[int, int]]:
+        """The [lo, hi) runs of the flat buffers (padding included) covered by the layout entries `indices`, each run
+        merging consecutive entries."""
+        runs: List[Tuple[int, int]] = []
+        for i in sorted(indices):
+            lo, hi = self.offsets[i], self.offsets[i] + self.padded_numel(i)
+            if runs and runs[-1][1] == lo:
+                runs[-1] = (runs[-1][0], hi)
+            else:
+                runs.append((lo, hi))
+        return runs
+
     # ---- gradient management -----------------------------------------------------------------------
     def zero_grad(self, set_to_none: bool = True) -> None:
         if set_to_none:
@@ -131,25 +143,20 @@ class FlatParameters:
         """Makes every existing `.grad` a view of the flat gradient buffer (copying the ones that live
         elsewhere, e.g. after a plain `loss.backward()`), and returns the [lo, hi) runs of the flat
         buffers covered by parameters that HAVE a gradient (torch optimizers skip the others)."""
-        dst, src = [], []
-        runs: List[Tuple[int, int]] = []
+        dst, src, have = [], [], []
         for i, p in enumerate(self.params):
             st = self.grad_state(p)
             if st == "none":
                 continue
+            have.append(i)
             if st == "other":
                 v = self._grad_views[i]
                 dst.append(v)
                 src.append(p.grad.detach().to(torch.float32).reshape(v.shape))
                 p.grad = v
-            lo, hi = self.offsets[i], self.offsets[i] + self.padded_numel(i)
-            if runs and runs[-1][1] == lo:
-                runs[-1] = (runs[-1][0], hi)
-            else:
-                runs.append((lo, hi))
         if dst:
             torch._foreach_copy_(dst, src)
-        return runs
+        return self.runs(have)
 
 
 def flat_plan(params: Sequence[Tensor]):

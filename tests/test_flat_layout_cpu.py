@@ -52,6 +52,7 @@ def test_gradient_adoption_runs_and_zero_grad(mv):
     assert flat.grad_state(ps[0]) == "other"
     runs = flat.gather_grads()
     assert runs == [(0, 144), (168, 172)]                                          # params 0-1 contiguous, param 3 alone
+    assert flat.runs([3, 0, 1]) == runs and flat.runs([]) == []
     assert flat.grad_state(ps[0]) == "view" and flat.grad_state(ps[2]) == "none"
     assert float(flat.flat_grad[:135].sum()) == 135.0 and float(flat.flat_grad[135]) == 0.0     # padding stays zero
     assert torch.equal(flat.flat_grad[136:141], torch.full((5,), 2.0)) and torch.equal(flat.flat_grad[168:171], torch.full((3,), 3.0))

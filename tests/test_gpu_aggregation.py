@@ -302,19 +302,26 @@ class _TinyMTL(torch.nn.Module):
         return f, [l1, l2, l3]
 
 
-@pytest.fixture(params=[False, True], ids=["sequential_rows", "batched_rows"])
-def jacobian_mode(request):
-    """Both ways of building the Jacobian rows: k sequential backward passes (default) and one vmapped pass."""
-    from movae_b200 import autojac
+@pytest.fixture(params=["segmented", "flat_jacobian"])
+def jacobian_mode(request, mv):
+    """Makes the test's aggregators for one of the engine's two paths: the segmented launch over the gradient tensors
+    (the default), or the flat J, forced by a forward hook on the weighting (hooks receive J).  `hooked` records the
+    hook calls."""
+    hooked = []
 
-    old = autojac.BATCHED_JACOBIAN
-    autojac.BATCHED_JACOBIAN = request.param
-    yield request.param
-    autojac.BATCHED_JACOBIAN = old
+    def make(name):
+        agg = mv.make_aggregator(name)
+        if request.param == "flat_jacobian":
+            agg.weighting.register_forward_hook(lambda m, inp, out: hooked.append(tuple(inp[0].shape)))
+        return agg
+
+    make.mode, make.hooked = request.param, hooked
+    return make
 
 
 @pytest.mark.parametrize("name", ["upgrad", "aligned_mtl", "mgda_ln"])
 def test_mtl_backward_and_backward_match_oracle(mv, oa, name, jacobian_mode):
+    make_aggregator = jacobian_mode
     torch.manual_seed(0)
     net = _TinyMTL().cuda()
     x = torch.randn(32, 7, device="cuda")
@@ -332,7 +339,7 @@ def test_mtl_backward_and_backward_match_oracle(mv, oa, name, jacobian_mode):
     # ---- mtl_backward ----------------------------------------------------------------------
     net.zero_grad(set_to_none=True)
     f, losses = net(x)
-    mv.mtl_backward(losses=losses, features=[f], aggregator=mv.make_aggregator(name), retain_graph=True)
+    mv.mtl_backward(losses=losses, features=[f], aggregator=make_aggregator(name), retain_graph=True)
     got = torch.cat([p.grad.flatten() for p in shared]).cpu()
     np.testing.assert_allclose(got.numpy(), g_ref.numpy(), rtol=RTOL, atol=ATOL)
     np.testing.assert_allclose(net.h1.weight.grad.cpu().numpy(), head_ref["h1"].cpu().numpy(), rtol=1e-5, atol=1e-7)
@@ -340,7 +347,7 @@ def test_mtl_backward_and_backward_match_oracle(mv, oa, name, jacobian_mode):
     np.testing.assert_allclose(net.code.grad.cpu().numpy(), head_ref["code"].cpu().numpy(), rtol=1e-5, atol=1e-7)
     # second call accumulates (torchjd Accumulate: += when .grad exists)
     f, losses = net(x)
-    mv.mtl_backward(losses=losses, features=[f], aggregator=mv.make_aggregator(name), retain_graph=True)
+    mv.mtl_backward(losses=losses, features=[f], aggregator=make_aggregator(name), retain_graph=True)
     got2 = torch.cat([p.grad.flatten() for p in shared]).cpu()
     np.testing.assert_allclose(got2.numpy(), 2 * g_ref.numpy(), rtol=RTOL, atol=2 * ATOL)
     # ---- backward over ALL parameters -------------------------------------------------------
@@ -352,9 +359,10 @@ def test_mtl_backward_and_backward_match_oracle(mv, oa, name, jacobian_mode):
         gs = torch.autograd.grad(l, params, retain_graph=True, allow_unused=True)
         rows.append(torch.cat([torch.zeros_like(p).flatten() if g is None else g.flatten() for p, g in zip(params, gs)]))
     _, _, g_all, _ = oa.aggregate(name, torch.stack(rows).cpu(), amtl_dtype=torch.float64)
-    mv.backward(losses, aggregator=mv.make_aggregator(name), inputs=params)
+    mv.backward(losses, aggregator=make_aggregator(name), inputs=params)
     got = torch.cat([p.grad.flatten() for p in params]).cpu()
     np.testing.assert_allclose(got.numpy(), g_all.numpy(), rtol=RTOL, atol=ATOL)
+    assert bool(jacobian_mode.hooked) == (jacobian_mode.mode == "flat_jacobian")      # the path under test ran
 
 
 # ------------------------------------------------------------------------------------ 8f "next" aggregators
